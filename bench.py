@@ -24,7 +24,10 @@ the step is config 4 of BASELINE.json: ONE univac-style cube (10 dimensions x 10
 scaling, fixed total cells — and a step rolls up an inner dimension (dim9 -> all, shard-local,
 HBM-bound) AND the sharded dimension (dim0 -> all: every rank computes its own output rows,
 reading the child rows out of its peers' stores over NVLink inside the rollup kernel).  A
-sharded-vs-single-cube parity guard runs on the devices before anything is timed."""
+sharded-vs-single-cube parity guard runs on the devices before anything is timed.
+
+  --dump-outputs DIR (N = 1): after the timed steps, the 4 result planes of the last one go to
+  DIR/<name>.npy, so that two builds can be compared output for output on identical inputs."""
 from __future__ import annotations
 
 import argparse
@@ -255,6 +258,15 @@ def sharded_config(world, ndims=None):
             "note": "N = 1 runs config 2 (the metric's own configuration); compare the N = 2, 4, 8 lines with one another"}
 
 
+def dump_outputs(directory, arrays):
+    """--dump-outputs: DIR/<name>.npy for every array the timed step hands its caller.  The inputs
+    come from synth() with fixed seeds, so two builds run with the same arguments can be compared
+    file by file.  Config 2 gives 4 float32 planes of 120 x 32^3 cells: 62.9 MB in all, written whole."""
+    os.makedirs(directory, exist_ok=True)
+    for name, arr in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), arr)
+
+
 # ------------------------------------------------------------------ GPU arm
 def run_ours(args, rank, world, local_rank):
     import torch
@@ -336,8 +348,9 @@ def run_ours(args, rank, world, local_rank):
         clocks.busy.set()
         with torch.cuda.stream(stream):
             e0.record(stream)
-            for _ in range(steps):
+            for _ in range(steps - 1):
                 fn()
+            timed.last = fn()  # the last step's results, for --dump-outputs
             e1.record(stream)
         barrier()
         clocks.busy.clear()
@@ -363,6 +376,13 @@ def run_ours(args, rank, world, local_rank):
     ms_value = timed(step_device, args.steps, args.warmup)
     launches = timed.launches  # kernels of libolapgpu.so launched inside the timed region
     N.check(lib.olap_set_async(0))
+    if args.dump_outputs:
+        rolled, ratio, _ = timed.last
+        outputs = {name: rolled.storedMeasures[name].data_f32() for name in names}
+        outputs["ratio"] = ratio.data_f32()
+        dump_outputs(args.dump_outputs, outputs)
+        del rolled, ratio, outputs
+    timed.last = None
 
     # per-launch duration of the dominant kernel, CUDA events on the launching stream
     step_device.measure = True
@@ -737,11 +757,18 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the result planes of the last timed step (m_sum, m_avg, m_max, ratio) as DIR/<name>.npy "
+                         "(float32); single GPU only")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or world > 1):
+        ap.error("--dump-outputs needs --impl ours on a single GPU")
     if args.impl == "reference":
         run_reference(args, rank)
         return
