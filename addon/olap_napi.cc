@@ -254,6 +254,51 @@ static napi_value Load(napi_env env, napi_callback_info info) {
     return nullptr;
 }
 
+// (Int32Array | null)[] -> item lists and their lengths; null = the whole axis
+static void region_lists(napi_env env, napi_value arr, const std::vector<int64_t>& lens,
+                         std::vector<const int32_t*>& ptrs, std::vector<int64_t>& keep_len) {
+    ptrs.assign(lens.size(), nullptr);
+    keep_len = lens;
+    for (uint32_t i = 0; i < (uint32_t)lens.size(); ++i) {
+        napi_value e;
+        napi_get_element(env, arr, i, &e);
+        bool typed = false;
+        napi_is_typedarray(env, e, &typed);
+        if (!typed) continue;
+        napi_typedarray_type t;
+        size_t len;
+        void* data;
+        napi_get_typedarray_info(env, e, &t, &len, &data, nullptr, nullptr);
+        ptrs[i] = static_cast<const int32_t*>(data);
+        keep_len[i] = (int64_t)len;
+    }
+}
+
+// regionSum(store, len[], keep (Int32Array|null)[]) -> number   (cube.js getTotalForDimensionItems)
+static napi_value RegionSum(napi_env env, napi_callback_info info) {
+    GET_ARGS();
+    auto len = int64_list(env, a.v[1]);
+    std::vector<const int32_t*> keep;
+    std::vector<int64_t> keep_len;
+    region_lists(env, a.v[2], len, keep, keep_len);
+    double v;
+    OLAP_CALL(olap_region_sum(unwrap(env, a.v[0]), (int)len.size(), len.data(), keep_len.data(), keep.data(), &v));
+    napi_value out;
+    NAPI_OK(napi_create_double(env, v, &out));
+    return out;
+}
+
+// regionCopy(dst, src, len[], keep (Int32Array|null)[])   (cube.js copyMeasureData)
+static napi_value RegionCopy(napi_env env, napi_callback_info info) {
+    GET_ARGS();
+    auto len = int64_list(env, a.v[2]);
+    std::vector<const int32_t*> keep;
+    std::vector<int64_t> keep_len;
+    region_lists(env, a.v[3], len, keep, keep_len);
+    OLAP_CALL(olap_region_copy(unwrap(env, a.v[0]), unwrap(env, a.v[1]), (int)len.size(), len.data(), keep_len.data(), keep.data()));
+    return nullptr;
+}
+
 // clone(store) -> external
 static napi_value Clone(napi_env env, napi_callback_info info) {
     GET_ARGS();
@@ -409,6 +454,8 @@ static napi_value Init(napi_env env, napi_value exports) {
         {"total", nullptr, Total, nullptr, nullptr, nullptr, napi_default, nullptr},
         {"drillDown", nullptr, DrillDown, nullptr, nullptr, nullptr, napi_default, nullptr},
         {"load", nullptr, Load, nullptr, nullptr, nullptr, napi_default, nullptr},
+        {"regionSum", nullptr, RegionSum, nullptr, nullptr, nullptr, napi_default, nullptr},
+        {"regionCopy", nullptr, RegionCopy, nullptr, nullptr, nullptr, napi_default, nullptr},
         {"clone", nullptr, Clone, nullptr, nullptr, nullptr, napi_default, nullptr},
         {"getValue", nullptr, GetValue, nullptr, nullptr, nullptr, napi_default, nullptr},
         {"setValue", nullptr, SetValue, nullptr, nullptr, nullptr, napi_default, nullptr},

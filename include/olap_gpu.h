@@ -264,6 +264,24 @@ int olap_reorder(olap_store* const* src, int n, int ndim, const int64_t* old_len
 int olap_load(olap_store* dst, const olap_store* src, int ndim, const int64_t* my_len, const int64_t* his_len,
               const int32_t* const* his_to_mine);
 
+/* ---- region queries (Cube.getTotalForDimensionItems / getDistribution / copyMeasureData, cube.js,
+ * which loop over the cartesian product of the filter's items with getSingleData / setSingleData).
+ * The region of a store of len[0] x ... x len[ndim-1] cells is keep[0] x ... x keep[ndim-1]:
+ * keep[d] = item indices of axis d (keep_len[d] of them), any order, repeats counted; keep[d] == NULL
+ * (or keep == NULL) = the whole axis in order.  One kernel (region/sum, region/copy); olap_last_op_ms()
+ * gives its time.  An empty region launches nothing. */
+/* getTotalForDimensionItems: double sum of the raw cells (unset = default) of the region
+ * keep[0] x ... x keep[ndim-1]; keep[d] = item indices of axis d, any order, repeats counted, NULL = whole axis.
+ * NaN cells (a NaN default's unset cells included) make the sum NaN.  Summation order is fixed for a
+ * given region: repeated calls give the same bits. */
+int olap_region_sum(const olap_store* s, int ndim, const int64_t* len, const int64_t* keep_len,
+                    const int32_t* const* keep, double* out);
+/* copyMeasureData: dst.setValue(i, src.getValue(i)) for every cell i of the region (dst, src same size):
+ * the source's raw value, canonicalised for dst's default, status byte SET / UNSET by dst's presence rule.
+ * dst may be src.  Cells outside the region are not touched. */
+int olap_region_copy(olap_store* dst, const olap_store* src, int ndim, const int64_t* len,
+                     const int64_t* keep_len, const int32_t* const* keep);
+
 /* ---- computed measures: Cube.getData(computedId) cube.js:331-363 --------------- */
 /* `program` is the formula in postfix text, space separated:
  *   v<k>  cell of input store k      t<k>  totals[k] (an `x__total` variable)

@@ -143,6 +143,12 @@ class GpuStore {
     native.load(this._h, other._h, lens(myDims), lens(hisDims), maps);
   }
 
+  // Region queries: a patched Cube.getTotalForDimensionItems / copyMeasureData lowers the filter to one
+  // item-index list per dimension (Int32Array, any order, repeats counted; null = the whole dimension)
+  // and makes ONE call instead of a getSingleData / setSingleData per combination (same lowering as store.py).
+  regionSum(len, keep) { return native.regionSum(this._h, len, keep); }
+  regionCopy(src, len, keep) { native.regionCopy(this._h, src._h, len, keep); }
+
   // Computed measures (cube.js:331-363): ONE fused kernel instead of a per-cell tree walk.
   // A patched Cube.getData(computedId) calls
   //   GpuStore.evaluate(expression, cellNames, cellNames.map((n) => this.storedMeasures[n]), totals, this.storeSize)

@@ -66,6 +66,13 @@ __global__ void __launch_bounds__(kStoreThreads) fill_kernel(float* __restrict__
     }
 }
 
+// setValue of one cell (in-memory.js:122-133): the canonical content of `x` and its status byte
+__device__ __forceinline__ float set_cell(float x, int nan_default, uint8_t& status) {
+    const float t = canon_store(x, nan_default);
+    status = present_f(t, nan_default) ? OLAP_STATUS_SET : OLAP_STATUS_UNSET;
+    return t;
+}
+
 // batched setValue (hydrateFromSparseNestedObject, setSingleData)
 __global__ void __launch_bounds__(kStoreThreads) set_values_kernel(float* __restrict__ v, uint8_t* __restrict__ st,
                                                                    const int64_t* __restrict__ idx,
@@ -77,9 +84,9 @@ __global__ void __launch_bounds__(kStoreThreads) set_values_kernel(float* __rest
     const int64_t k = idx[i];
     if (k < 0 || k >= size) return;
     if (lossy && val[i] == val[i] && (double)(float)val[i] != val[i]) atomicMin(lossy, (unsigned long long)i + 1);
-    const float t = canon_store((float)val[i], nan_default);
-    v[k] = t;
-    if (st) st[k] = present_f(t, nan_default) ? OLAP_STATUS_SET : OLAP_STATUS_UNSET;
+    uint8_t s;
+    v[k] = set_cell((float)val[i], nan_default, s);
+    if (st) st[k] = s;
 }
 
 __device__ __forceinline__ double warp_sum(double x) {

@@ -21,6 +21,7 @@
 #include "kernels_long.cuh"
 #include "kernels_lanes.cuh"
 #include "kernels_pull.cuh"
+#include "kernels_region.cuh"
 #include "kernels_tma.cuh"
 #include "host_pipe.cuh"
 
@@ -1845,6 +1846,174 @@ int olap_load(olap_store* dst, const olap_store* src, int ndim, const int64_t* m
         OLAP_TRY(t.release());
     }
     end_op("load/scatter");
+    return finish_op();
+}
+
+// ---- region queries: getTotalForDimensionItems / copyMeasureData -------------------------
+namespace {
+
+// The region keep[0] x ... x keep[ndim-1] of a store of len[0] x ... x len[ndim-1] cells, lowered like a
+// dice (olap_dice): an identity list becomes a stride, any other list an int64 offset table; one-item axes
+// fold into a constant offset, whole neighbours merge, and the trailing whole axes form the inner run.
+struct RegionPlan {
+    std::vector<GDim> dims;   // outer axes (tables or strides)
+    int64_t const_off = 0, I = 1, cells = 0;
+};
+
+static int plan_region(const char* what, int64_t size, int ndim, const int64_t* len, const int64_t* keep_len,
+                       const int32_t* const* keep, RegionPlan* plan) {
+    if (ndim < 0 || ndim > OLAP_MAX_DIMS) return fail(OLAP_E_INVALID, "%s: at most %d dimensions", what, OLAP_MAX_DIMS);
+    if (ndim && !len) return fail(OLAP_E_INVALID, "%s: null argument", what);
+    int64_t total = 0;
+    OLAP_TRY(product(len, ndim, &total, what));
+    if (total != size) return fail(OLAP_E_INVALID, "%s: dimensions describe %lld cells, store has %lld", what, (long long)total, (long long)size);
+    std::vector<int64_t> n(ndim);
+    for (int d = 0; d < ndim; ++d) {
+        const bool whole = !keep || !keep[d];
+        if (!whole && (!keep_len || keep_len[d] < 0)) return fail(OLAP_E_INVALID, "%s: dimension %d has no list length", what, d);
+        n[d] = whole ? len[d] : keep_len[d];
+    }
+    OLAP_TRY(product(n.data(), ndim, &plan->cells, what));
+    plan->dims.assign(ndim, GDim{});
+    int64_t stride = 1;
+    for (int d = ndim - 1; d >= 0; --d) {
+        GDim& g_ = plan->dims[d];
+        g_.len = n[d];
+        bool identity = n[d] == len[d];
+        if (keep && keep[d])
+            for (int64_t j = 0; j < n[d]; ++j) {
+                const int32_t o = keep[d][j];
+                if (o < 0 || o >= len[d]) return fail(OLAP_E_INVALID, "%s: dimension %d lists item %d, outside [0, %lld)", what, d, o, (long long)len[d]);
+                identity &= o == j;
+            }
+        if (identity) { g_.linear = true; g_.stride = stride; }
+        else {
+            g_.linear = false;
+            g_.tbl.resize(n[d]);
+            for (int64_t j = 0; j < n[d]; ++j) g_.tbl[j] = (int64_t)keep[d][j] * stride;
+        }
+        stride *= len[d];
+    }
+    if (plan->cells == 0) return OLAP_OK;
+    merge_dims(plan->dims, &plan->const_off);
+    if (!plan->dims.empty() && plan->dims.back().linear && plan->dims.back().stride == 1) {
+        plan->I = plan->dims.back().len;
+        plan->dims.pop_back();
+    }
+    if ((int)plan->dims.size() > OLAP_MAX_DIMS) return fail(OLAP_E_UNSUPPORTED, "%s: too many dimensions", what);
+    for (auto& d : plan->dims)
+        if (d.len > 0xffffffffLL) return fail(OLAP_E_UNSUPPORTED, "%s: merged dimension longer than 2^32-1", what);
+    return OLAP_OK;
+}
+
+// 128-bit accesses when the inner run, every offset and the planes allow them
+static int region_vec(const RegionPlan& plan, const void* a, const void* b, const void* st) {
+    if (plan.I % 4 || plan.const_off % 4) return 1;
+    if ((reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(b)) & 15) return 1;
+    if (reinterpret_cast<uintptr_t>(st) & 3) return 1;
+    for (auto& d : plan.dims) {
+        if (d.linear) { if (d.stride % 4) return 1; }
+        else for (int64_t v : d.tbl) if (v % 4) return 1;
+    }
+    return 4;
+}
+
+// Tables to the device, index fields of p.ix; returns the grid
+static int region_params(const RegionPlan& plan, int VEC, TablePack& t, RegionParams& p) {
+    std::vector<size_t> o_tbl(plan.dims.size(), 0);
+    int64_t rows = 1;
+    for (size_t d = 0; d < plan.dims.size(); ++d) {
+        if (!plan.dims[d].linear) o_tbl[d] = t.add(plan.dims[d].tbl.data(), plan.dims[d].tbl.size() * 8);
+        rows *= plan.dims[d].len;
+    }
+    OLAP_TRY(t.upload());
+    GatherParams& q = p.ix;
+    q.nd = (int)plan.dims.size();
+    for (size_t d = 0; d < plan.dims.size(); ++d) {
+        q.len[d] = (uint32_t)plan.dims[d].len;
+        q.div[d] = FastDiv((uint32_t)plan.dims[d].len);
+        q.tbl[d] = plan.dims[d].linear ? nullptr : t.ptr<int64_t>(o_tbl[d]);
+        q.lin[d] = plan.dims[d].stride;
+    }
+    const int64_t IV = plan.I / VEC;
+    q.I = plan.I;
+    q.rows = rows;
+    q.n_vec = rows * IV;
+    p.big = q.n_vec >= ((int64_t)1 << 31) || IV > 0xffffffffLL;
+    for (auto& d : plan.dims) p.big |= d.len >= ((int64_t)1 << 31);
+    if (IV > 0xffffffffLL) return fail(OLAP_E_UNSUPPORTED, "region: inner run too long");
+    q.IV = (uint32_t)IV;
+    q.div_iv = FastDiv(p.big ? 1u : (uint32_t)IV);
+    return OLAP_OK;
+}
+
+}  // namespace
+
+int olap_region_sum(const olap_store* s, int ndim, const int64_t* len, const int64_t* keep_len,
+                    const int32_t* const* keep, double* out) {
+    if (!s || !out) return fail(OLAP_E_INVALID, "olap_region_sum: null argument");
+    RegionPlan plan;
+    OLAP_TRY(plan_region("olap_region_sum", s->size, ndim, len, keep_len, keep, &plan));
+    OLAP_TRY(ensure_ctx());
+    *out = 0.0;
+    begin_op();
+    if (plan.cells == 0) {
+        end_op("region/sum");
+        return finish_op();
+    }
+    const int VEC = region_vec(plan, s->values + plan.const_off, s->values + plan.const_off, nullptr);
+    RegionParams p{};
+    TablePack t;
+    OLAP_TRY(region_params(plan, VEC, t, p));
+    const int blocks = grid_for(p.ix.n_vec, 256);
+    void* scratch;
+    OLAP_TRY(dev_alloc(&scratch, (size_t)blocks * 8 + 16));
+    p.src = s->values + plan.const_off;
+    p.partial = static_cast<double*>(scratch);
+    p.out = p.partial + blocks;
+    p.ticket = reinterpret_cast<unsigned int*>(p.out + 1);
+    OLAP_CUDA(cudaMemsetAsync(p.ticket, 0, 4, g.stream));
+    KERNELS_BEGIN();
+    if (VEC == 4) region_kernel<REGION_SUM, 4><<<blocks, 256, 0, g.stream>>>(p);
+    else region_kernel<REGION_SUM, 1><<<blocks, 256, 0, g.stream>>>(p);
+    LAUNCHED();
+    end_op("region/sum");
+    double host = 0.0;
+    OLAP_CUDA(cudaMemcpyAsync(&host, p.out, 8, cudaMemcpyDeviceToHost, g.stream));
+    OLAP_TRY(t.release());
+    OLAP_TRY(dev_free(scratch));
+    OLAP_CUDA(cudaStreamSynchronize(g.stream));
+    *out = host;
+    return finish_op();
+}
+
+int olap_region_copy(olap_store* dst, const olap_store* src, int ndim, const int64_t* len, const int64_t* keep_len,
+                     const int32_t* const* keep) {
+    if (!dst || !src) return fail(OLAP_E_INVALID, "olap_region_copy: null store");
+    if (dst->size != src->size) return fail(OLAP_E_INVALID, "olap_region_copy: stores of %lld and %lld cells", (long long)dst->size, (long long)src->size);
+    RegionPlan plan;
+    OLAP_TRY(plan_region("olap_region_copy", src->size, ndim, len, keep_len, keep, &plan));
+    OLAP_TRY(ensure_ctx());
+    begin_op();
+    // the derived flag stays as it is, as for olap_store_set_values: every byte written is  set ? SET : UNSET
+    if (plan.cells) {
+        const int VEC = region_vec(plan, src->values + plan.const_off, dst->values + plan.const_off,
+                                   dst->status ? dst->status + plan.const_off : nullptr);
+        RegionParams p{};
+        TablePack t;
+        OLAP_TRY(region_params(plan, VEC, t, p));
+        p.src = src->values + plan.const_off;
+        p.dst = dst->values + plan.const_off;
+        p.st_dst = dst->status ? dst->status + plan.const_off : nullptr;
+        p.dst_nan_default = dst->default_kind;
+        const int blocks = grid_for(p.ix.n_vec, 256);
+        KERNELS_BEGIN();
+        if (VEC == 4) region_kernel<REGION_COPY, 4><<<blocks, 256, 0, g.stream>>>(p);
+        else region_kernel<REGION_COPY, 1><<<blocks, 256, 0, g.stream>>>(p);
+        LAUNCHED();
+        OLAP_TRY(t.release());
+    }
+    end_op("region/copy");
     return finish_op();
 }
 

@@ -49,6 +49,106 @@ def _check_measure_id(measureId):
         raise ValueError(f"Invalid measureId: {measureId}")
 
 
+def _check_coords(dimensions, who, coords):
+    ids = [d.id for d in dimensions]
+    if any(not coords.get(d) for d in ids):
+        raise ValueError(f"{who}: no value for all dimensions. Dimensions: {','.join(ids)}, Coords: {coords}")
+
+
+def _position(dimensions, coords):
+    position = 0
+    for dimension in dimensions:
+        if dimension.id not in coords:
+            raise ValueError(f"getPosition: no such dimension {dimension.id}. Coords: {coords}")
+        index = dimension.getRootIndexFromRootItem(coords[dimension.id])
+        if index == -1:
+            raise ValueError(f"getPosition: no such item {coords[dimension.id]}. Dimension items: {dimension.getItems()}")
+        position = position * dimension.numItems + index
+    return position
+
+
+def _check_readable(storedMeasures, computedMeasures, measureId):
+    """What getSingleData(measureId, coords) raises for a measure, once the coordinates are valid."""
+    if measureId in storedMeasures:
+        return
+    if measureId in computedMeasures:
+        for name in computedMeasures[measureId].variables():
+            if name not in storedMeasures:
+                raise KeyError(name)  # an `x__total` variable: the per-cell evaluation has no such store
+        return
+    raise KeyError(f"getSingleData: no such measure {measureId}")
+
+
+def _region(dimensions, dimensionsFilter, check_measures):
+    """The combinations of getTotalForDimensionItems / copyMeasureData (cube.js) as one region of the store:
+    (lens, keep), keep[d] = item indices of dimension d in filter order, repeats kept, or None for a dimension
+    the filter does not name.  A filter key that is not a dimension multiplies every combination by the length
+    of its list: a leading axis of one item listed that many times.  None when there is no combination.
+
+    Raises what the loop raises on its first failing combination, in its order (filter keys in dict order,
+    then the other dimensions, last key fastest); `check_measures` raises what every valid combination would."""
+    options = {k: ([v] if isinstance(v, str) else list(v)) for k, v in (dimensionsFilter or {}).items()}
+    for d in dimensions:
+        if d.id not in options:
+            options[d.id] = None
+    keys = list(options)
+    by_id = {d.id: d for d in dimensions}
+    if any((by_id[k].numItems if v is None else len(v)) == 0 for k, v in options.items()):
+        return None
+
+    def bad(key, item):
+        return key in by_id and (not item or by_id[key].getRootIndexFromRootItem(item) == -1)
+
+    def first_item(key):
+        return options[key][0] if options[key] is not None else by_id[key].getItems()[0]
+
+    def fail(combination):
+        _check_coords(dimensions, "getSingleData", combination)
+        _position(dimensions, combination)
+
+    first = {k: first_item(k) for k in keys}
+    if any(bad(k, v) for k, v in first.items()):
+        fail(first)
+    check_measures()
+    # the first failing combination differs from the first one in ONE key: the fastest-varying key that has a bad item
+    for k in reversed(keys):
+        if options[k] is None:
+            continue
+        for item in options[k]:
+            if bad(k, item):
+                fail({**first, k: item})
+    lens, keep = [d.numItems for d in dimensions], []
+    for d in dimensions:
+        items = options[d.id]
+        keep.append(None if items is None else np.array([d.getRootIndexFromRootItem(i) for i in items], dtype=np.int32))
+    multiplicity = 1
+    for k in keys:
+        if k not in by_id:
+            multiplicity *= len(options[k])
+    if multiplicity != 1:
+        lens, keep = [1] + lens, [np.zeros(multiplicity, dtype=np.int32)] + keep
+    return lens, keep
+
+
+def _region_lists(lens, keep):
+    return [np.arange(n) if k is None else np.asarray(k, dtype=np.int64) for n, k in zip(lens, keep)]
+
+
+def _region_sum_f64(data, lens, keep):
+    """Region sum of a computed measure evaluated on the host (doubles)."""
+    return float(data.reshape(lens)[np.ix_(*_region_lists(lens, keep))].sum())
+
+
+def _region_set_f64(store, data, lens, keep):
+    """store.setValue(i, data[i]) for every cell i of the region (a computed source): one batched call."""
+    index = np.ravel_multi_index(np.ix_(*_region_lists(lens, keep)), lens).ravel() if lens else np.zeros(1, np.int64)
+    if hasattr(store, "setValues"):
+        store.setValues(index, data[index])
+    else:
+        for i in index.tolist():
+            store.setValue(i, float(data[i]))
+
+
 class Cube:
     def __init__(self, dimensions, store_cls=None):
         self.dimensions = list(dimensions)
@@ -337,10 +437,7 @@ class Cube:
                 self._collect_sparse(child, offset * dimension.numItems + item_offset, dimOffset + 1, indexes, values)
 
     def _check_coords(self, who, coords):
-        if any(not coords.get(d) for d in self.dimensionIds):
-            raise ValueError(
-                f"{who}: no value for all dimensions. Dimensions: {','.join(self.dimensionIds)}, Coords: {coords}"
-            )
+        _check_coords(self.dimensions, who, coords)
 
     def setSingleData(self, measureId, coords, value):
         self._check_coords("setSingleData", coords)
@@ -360,17 +457,7 @@ class Cube:
         raise KeyError(f"getSingleData: no such measure {measureId}")
 
     def getPosition(self, coords):
-        position = 0
-        for dimension in self.dimensions:
-            if dimension.id not in coords:
-                raise ValueError(f"getPosition: no such dimension {dimension.id}. Coords: {coords}")
-            index = dimension.getRootIndexFromRootItem(coords[dimension.id])
-            if index == -1:
-                raise ValueError(
-                    f"getPosition: no such item {coords[dimension.id]}. Dimension items: {dimension.getItems()}"
-                )
-            position = position * dimension.numItems + index
-        return position
+        return _position(self.dimensions, coords)
 
     def getTotal(self, measureId):
         return self.storedMeasures[measureId].total
@@ -383,12 +470,19 @@ class Cube:
         keys = list(options.keys())
         return [dict(zip(keys, combo)) for combo in itertools.product(*[options[k] for k in keys])]
 
+    # getTotalForDimensionItems / copyMeasureData: the reference loops over every combination of the
+    # filter's items with getSingleData / setSingleData.  Here the combinations are one region of the
+    # store (per-dimension item lists, _region) and one store call covers it; results and errors are
+    # those of the loop.
     def getTotalForDimensionItems(self, measureId, dimensionsFilter=None):
-        options = {k: ([v] if isinstance(v, str) else v) for k, v in (dimensionsFilter or {}).items()}
-        for d in self.dimensionIds:
-            if d not in options:
-                options[d] = self.getDimension(d).getItems()
-        return sum((self.getSingleData(measureId, c) for c in self._combinations(options)), 0)
+        region = _region(self.dimensions, dimensionsFilter,
+                         lambda: _check_readable(self.storedMeasures, self.computedMeasures, measureId))
+        if region is None:
+            return 0
+        lens, keep = region
+        if measureId in self.storedMeasures:
+            return self.storedMeasures[measureId].regionSum(lens, keep)
+        return _region_sum_f64(np.asarray(self.getData(measureId), dtype=np.float64), lens, keep)
 
     def getDistribution(self, measureId, dimensionsFilter=None):
         space = self.getTotalForDimensionItems(measureId, dimensionsFilter)
@@ -396,12 +490,20 @@ class Cube:
         return space if total == 0 else space / total
 
     def copyMeasureData(self, sourceMeasureId, targetMeasureId, dimensionsFilter=None):
-        options = {k: ([v] if isinstance(v, str) else v) for k, v in (dimensionsFilter or {}).items()}
-        for d in self.dimensionIds:
-            if d not in options:
-                options[d] = self.getDimension(d).getItems()
-        for combination in self._combinations(options):
-            self.setSingleData(targetMeasureId, combination, self.getSingleData(sourceMeasureId, combination))
+        def check():
+            _check_readable(self.storedMeasures, self.computedMeasures, sourceMeasureId)
+            if targetMeasureId not in self.storedMeasures:
+                raise ValueError(f"setSingleData: no such stored measure {targetMeasureId}")
+
+        region = _region(self.dimensions, dimensionsFilter, check)
+        if region is None:
+            return
+        lens, keep = region
+        target = self.storedMeasures[targetMeasureId]
+        if sourceMeasureId in self.storedMeasures:
+            target.regionCopy(self.storedMeasures[sourceMeasureId], lens, keep)
+        else:
+            _region_set_f64(target, np.asarray(self.getData(sourceMeasureId), dtype=np.float64), lens, keep)
 
     def scan(self, dimensionIds, cb):
         for combination in self._combinations(self.getDimensionItemsMap(dimensionIds)):

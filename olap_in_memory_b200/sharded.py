@@ -24,6 +24,7 @@ import os
 
 import numpy as np
 
+from . import cube as _cube
 from .cube import Cube  # noqa: F401  (re-exported for convenience)
 
 
@@ -418,6 +419,57 @@ class ShardedCube:
         store = self.storedMeasures[measureId]
         device = self._store_cls.DEVICE if self.world > 1 else None
         return self.comm.all_reduce_sum(store.total, device)
+
+    # ------------------------------------------------------------ region queries
+    def _local_region(self, dimensionsFilter, check_measures):
+        """Cube._region on the whole cube (the same validation and errors on every rank, before any collective),
+        restricted to my rows: the filter lists of the row dimensions (and the leading multiplicity axis of filter
+        keys that are not dimensions) give global rows in product order, repeats kept; those in [row0, row1) are
+        the first-axis list of my region.  None when the whole region is empty."""
+        region = _cube._region(self.dimensions, dimensionsFilter, check_measures)
+        if region is None:
+            return None
+        lens, keep = region
+        lead = len(lens) - len(self.dimensions) + self.prefix  # row axes, the multiplicity axis included
+        rows = np.ravel_multi_index(np.ix_(*_cube._region_lists(lens[:lead], keep[:lead])), lens[:lead]).ravel()
+        mine = rows[(rows >= self.row0) & (rows < self.row1)] - self.row0
+        return [self.rows_local] + self.inner_lens, [mine.astype(np.int32)] + keep[lead:]
+
+    def getTotalForDimensionItems(self, measureId, dimensionsFilter=None):
+        """Cube.getTotalForDimensionItems: the region sum of my rows, then one all-reduce that every rank joins."""
+        region = self._local_region(dimensionsFilter,
+                                    lambda: _cube._check_readable(self.storedMeasures, self.computedMeasures, measureId))
+        if region is None:
+            return 0
+        lens, keep = region
+        if measureId in self.storedMeasures:
+            local = self.storedMeasures[measureId].regionSum(lens, keep)
+        else:
+            local = _cube._region_sum_f64(np.asarray(self.getLocalData(measureId), dtype=np.float64), lens, keep)
+        device = self._store_cls.DEVICE if self.world > 1 else None
+        return self.comm.all_reduce_sum(float(local), device)
+
+    def getDistribution(self, measureId, dimensionsFilter=None):
+        space = self.getTotalForDimensionItems(measureId, dimensionsFilter)
+        total = self.getTotal(measureId)
+        return space if total == 0 else space / total
+
+    def copyMeasureData(self, sourceMeasureId, targetMeasureId, dimensionsFilter=None):
+        """Cube.copyMeasureData on my rows: both measures have the same row bounds, nothing crosses ranks."""
+        def check():
+            _cube._check_readable(self.storedMeasures, self.computedMeasures, sourceMeasureId)
+            if targetMeasureId not in self.storedMeasures:
+                raise ValueError(f"setSingleData: no such stored measure {targetMeasureId}")
+
+        region = self._local_region(dimensionsFilter, check)
+        if region is None or region[1][0].size == 0:
+            return
+        lens, keep = region
+        target = self.storedMeasures[targetMeasureId]
+        if sourceMeasureId in self.storedMeasures:
+            target.regionCopy(self.storedMeasures[sourceMeasureId], lens, keep)
+        else:
+            _cube._region_set_f64(target, np.asarray(self.getLocalData(sourceMeasureId), dtype=np.float64), lens, keep)
 
     @staticmethod
     def _set(store, values):

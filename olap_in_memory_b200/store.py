@@ -234,6 +234,28 @@ class GpuStore:
         )
         del keep
 
+    # ---- region queries (Cube.getTotalForDimensionItems / copyMeasureData) -------------
+    @staticmethod
+    def _region_args(lens, keep):
+        """keep[d]: item indices of axis d (any order, repeats counted) or None for the whole axis."""
+        alive, ptrs = N.map_arrays(keep)
+        keep_len = [n if k is None else len(k) for n, k in zip(lens, alive)]
+        return alive, len(lens), N.i64_array(lens), N.i64_array(keep_len), ptrs
+
+    def regionSum(self, lens, keep):
+        """Double sum of the raw cells (unset cells count as the default) of keep[0] x ... x keep[-1]."""
+        alive, nd, len_arr, keep_len, ptrs = self._region_args(lens, keep)
+        out = C.c_double()
+        N.check(N.lib().olap_region_sum(self._h, nd, len_arr, keep_len, ptrs, C.byref(out)))
+        del alive
+        return out.value
+
+    def regionCopy(self, src, lens, keep):
+        """self.setValue(i, src.getValue(i)) for every cell i of keep[0] x ... x keep[-1], in place."""
+        alive, nd, len_arr, keep_len, ptrs = self._region_args(lens, keep)
+        N.check(N.lib().olap_region_copy(self._h, src._h, nd, len_arr, keep_len, ptrs))
+        del alive
+
     # ---- single-store forms of the transforms ------------------------------------
     def reorder(self, oldDimensions, newDimensions):
         return GpuStore.reorder_many([self], oldDimensions, newDimensions)[0]
