@@ -679,6 +679,15 @@ struct ScatterParams {
     int64_t n;
 };
 
+// Status byte of a cell load writes: "status flags are copied between cubes" (README.md:704), but whether the cell
+// is set follows MY default.  A set cell takes the source's byte when that byte says set, else SET: a zero-default
+// source's unset 0 (0x1) is a set cell of a NaN-default target, and a plane that says UNSET there would no longer
+// follow from the values (olap_store::derived).
+__device__ __forceinline__ uint32_t load_status(bool set, uint32_t src_byte) {
+    if (!set) return OLAP_STATUS_UNSET;
+    return (src_byte & OLAP_STATUS_SET) ? src_byte : (uint32_t)OLAP_STATUS_SET;
+}
+
 static __global__ void __launch_bounds__(256) load_scatter_kernel(const __grid_constant__ ScatterParams p) {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= p.n) return;
@@ -698,9 +707,7 @@ static __global__ void __launch_bounds__(256) load_scatter_kernel(const __grid_c
     p.dst[off] = canon_store(v, p.dst_nan_default);
     if (p.st_dst) {
         const bool set = present_f(canon_store(v, p.dst_nan_default), p.dst_nan_default);
-        uint8_t s = set ? OLAP_STATUS_SET : OLAP_STATUS_UNSET;
-        if (p.st_src && set) s = p.st_src[t];  // "status flags are copied between cubes" README.md:704
-        p.st_dst[off] = s;
+        p.st_dst[off] = load_status(set, p.st_src ? p.st_src[t] : (uint32_t)OLAP_STATUS_SET);
     }
 }
 
@@ -756,9 +763,7 @@ __global__ void __launch_bounds__(256) load_scatter_vec_kernel(const __grid_cons
     for (int e = 0; e < VEC; ++e) {
         v[e] = canon_store(v[e], p.dst_nan_default);
         const bool set = present_f(v[e], p.dst_nan_default);
-        uint32_t sx = set ? (uint32_t)OLAP_STATUS_SET : (uint32_t)OLAP_STATUS_UNSET;
-        if (p.st_src && set) sx = (sb >> (8 * e)) & 0xffu;  // "status flags are copied between cubes" README.md:704
-        so |= sx << (8 * e);
+        so |= load_status(set, p.st_src ? (sb >> (8 * e)) & 0xffu : (uint32_t)OLAP_STATUS_SET) << (8 * e);
     }
     if (VEC == 4) {
         st_stream4(p.dst + off, make_float4(v[0], v[1 % VEC], v[2 % VEC], v[3 % VEC]));

@@ -509,14 +509,23 @@ static int launch_down_mid(const DownMeasure* d_meas, int n, const Csr& csr, con
     return OLAP_OK;
 }
 
+// The block kernel's dynamic shared memory: RB rows of P * I staged parent cells (step, result, status, truthy:
+// 14 bytes each), the [C] parent and rank tables, and 16 bytes of alignment.  It opts in to kDownBlockSmem bytes.
+constexpr size_t kDownBlockSmem = 160 * 1024;
+static int64_t down_block_rows(int64_t O, int64_t C, int64_t I) { return std::max<int64_t>(1, std::min<int64_t>(O, 8192 / (C * I))); }
+static size_t down_block_smem(int64_t O, int64_t P, int64_t C, int64_t I) {
+    return (size_t)down_block_rows(O, C, I) * P * I * (8 + 4 + 1 + 1) + (size_t)C * 8 + 16;
+}
+
 // The block kernel stages P * I parent cells (14 bytes each) of at least one outer index in shared memory.
 // With an inner run behind the drilled axis the integer-spreading measures stay on the parent-driven
 // kernel, which carries floor((k - 1) * step) from child to child (the block kernel would redo both
-// floors per cell: 0.38 against 0.64 of peak).
-static bool down_block_fits(int64_t P, int64_t C, int64_t I, bool any_int = false) {
+// floors per cell: 0.38 against 0.64 of peak).  Shapes whose staging exceeds kDownBlockSmem (long rows, or
+// many parents without children) take the mid or gather kernels.
+static bool down_block_fits(int64_t O, int64_t P, int64_t C, int64_t I, bool any_int = false) {
     static const int knob = [] { const char* e = getenv("OLAP_DOWN_BLOCK"); return e ? atoi(e) : 1; }();
-    if (I == 1) return C <= 8192 && P <= 8192;
-    return knob && !any_int && P * I <= 8192 && C <= 8192 && C * I < (1 << 28) && I <= 2048;
+    bool fits = I == 1 ? C <= 8192 && P <= 8192 : knob && !any_int && P * I <= 8192 && C <= 8192 && C * I < (1 << 28) && I <= 2048;
+    return fits && down_block_smem(O, P, C, I) <= kDownBlockSmem;
 }
 
 static int launch_down_inner(const DownMeasure* d_meas, int n, const int32_t* d_parent, const int32_t* d_rank,
@@ -527,17 +536,17 @@ static int launch_down_inner(const DownMeasure* d_meas, int n, const int32_t* d_
     p.rank_of = d_rank;
     p.cnt_of = d_cnt;
     p.O = O; p.P = (int32_t)P; p.C = (int32_t)C; p.I = (uint32_t)I;
-    p.RB = (uint32_t)std::max<int64_t>(1, std::min<int64_t>(O, 8192 / (C * I)));
+    p.RB = (uint32_t)down_block_rows(O, C, I);
     p.vec4 = I == 1 ? (C % 4 == 0 && ((int64_t)p.RB * C) % 4 == 0) : (I % 4 == 0);
     p.div_i = FastDiv((uint32_t)I);
     p.div_pi = FastDiv((uint32_t)(P * I));
     p.div_ci = FastDiv((uint32_t)(C * I));
-    const size_t smem = (size_t)p.RB * P * I * (8 + 4 + 1 + 1) + (size_t)C * 8 + 16;
+    const size_t smem = down_block_smem(O, P, C, I);
     const int64_t gx = ceil_div(O, p.RB);
     if (gx > 0x7fffffffLL) return fail(OLAP_E_UNSUPPORTED, "drillDown: grid too large");
     static bool attr = false;
     if (!attr) {
-        OLAP_CUDA(cudaFuncSetAttribute(drilldown_inner_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
+        OLAP_CUDA(cudaFuncSetAttribute(drilldown_inner_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kDownBlockSmem));
         attr = true;
     }
     KERNELS_BEGIN();
@@ -1631,6 +1640,10 @@ int olap_drill_down(olap_store* const* src, int n, const int* methods, int ndim,
     bool any_int_sum = false;
     for (int k = 0; k < n; ++k)
         any_int_sum |= (src[k]->type == OLAP_INT32 || src[k]->type == OLAP_UINT32) && (methods ? methods[k] == OLAP_SUM : true);
+    int64_t O_changed = 1;  // cells in front of the changed dimension when there is one
+    for (int q = 0; changed.size() == 1 && q < changed[0]; ++q) O_changed *= old_len[q];
+    const bool block = new_size && !any_dist && changed.size() == 1 &&
+                       down_block_fits(O_changed, old_len[changed[0]], new_len[changed[0]], inner_of_changed, any_int_sum);
     OLAP_TRY(ensure_ctx());
     OLAP_TRY(alloc_like(src, n, new_size, out));
     OutGuard guard(out, n);
@@ -1639,7 +1652,7 @@ int olap_drill_down(olap_store* const* src, int n, const int* methods, int ndim,
     int rc = OLAP_OK;
     if (new_size && old_size == 0) {
         for (int k = 0; k < n; ++k) { olap_store t = *out[k]; t.status = st_out_of(out, k); OLAP_TRY(fill_default(&t)); }
-    } else if (new_size && !any_dist && changed.size() == 1 && !down_block_fits(old_len[changed[0]], new_len[changed[0]], inner_of_changed, any_int_sum) &&
+    } else if (new_size && !any_dist && changed.size() == 1 && !block &&
                ((inner_of_changed % 4 == 0 && inner_of_changed >= 32) || (inner_of_changed % 2 == 0 && inner_of_changed >= 64) ||
                 inner_of_changed >= 128)) {
         // one changed dimension with a long inner run: parent-driven kernel
@@ -1667,7 +1680,7 @@ int olap_drill_down(olap_store* const* src, int n, const int* methods, int ndim,
         OLAP_TRY(launch_down_mid(t.ptr<DownMeasure>(o_meas), n, csr, t.ptr<int32_t>(o_ps), t.ptr<int32_t>(o_ch), O,
                                  old_len[d], new_len[d], inner_of_changed, kind));
         OLAP_TRY(t.release());
-    } else if (new_size && !any_dist && changed.size() == 1 && down_block_fits(old_len[changed[0]], new_len[changed[0]], inner_of_changed, any_int_sum)) {
+    } else if (block) {
         // the drilled dimension is the innermost one, or the run behind it is short: block kernel,
         // parents staged in shared memory, output written front to back with 128-bit stores
         const int d = changed[0];
