@@ -443,6 +443,84 @@ static napi_value EvaluateToStore(napi_env env, napi_callback_info info) {
     return wrap_store(env, s);
 }
 
+// program string argument -> NUL-terminated buffer
+static napi_status utf8_arg(napi_env env, napi_value v, std::vector<char>& out) {
+    size_t plen = 0;
+    const napi_status st = napi_get_value_string_utf8(env, v, nullptr, 0, &plen);
+    if (st != napi_ok) return st;
+    out.assign(plen + 1, '\0');
+    return napi_get_value_string_utf8(env, v, out.data(), out.size(), &plen);
+}
+
+// regionEvalSum(program string, stores[], len[], keep (Int32Array|null)[]) -> number
+//   (getTotalForDimensionItems of a computed measure)
+static napi_value RegionEvalSum(napi_env env, napi_callback_info info) {
+    GET_ARGS();
+    std::vector<char> program;
+    NAPI_OK(utf8_arg(env, a.v[0], program));
+    auto src = store_list(env, a.v[1]);
+    auto len = int64_list(env, a.v[2]);
+    std::vector<const int32_t*> keep;
+    std::vector<int64_t> keep_len;
+    region_lists(env, a.v[3], len, keep, keep_len);
+    double v;
+    OLAP_CALL(olap_region_eval_sum(program.data(), src.data(), (int)src.size(), (int)len.size(), len.data(), keep_len.data(),
+                                   keep.data(), &v));
+    napi_value out;
+    NAPI_OK(napi_create_double(env, v, &out));
+    return out;
+}
+
+// regionEvalCopy(dst, program string, stores[], len[], keep (Int32Array|null)[])   (copyMeasureData, computed source)
+static napi_value RegionEvalCopy(napi_env env, napi_callback_info info) {
+    GET_ARGS();
+    std::vector<char> program;
+    NAPI_OK(utf8_arg(env, a.v[1], program));
+    auto src = store_list(env, a.v[2]);
+    auto len = int64_list(env, a.v[3]);
+    std::vector<const int32_t*> keep;
+    std::vector<int64_t> keep_len;
+    region_lists(env, a.v[4], len, keep, keep_len);
+    OLAP_CALL(olap_region_eval_copy(unwrap(env, a.v[0]), program.data(), src.data(), (int)src.size(), (int)len.size(), len.data(),
+                                    keep_len.data(), keep.data()));
+    return nullptr;
+}
+
+// statusMerge(stores[], Uint8Array)   (getStatus of a computed measure)
+static napi_value StatusMerge(napi_env env, napi_callback_info info) {
+    GET_ARGS();
+    auto src = store_list(env, a.v[0]);
+    napi_typedarray_type t;
+    size_t len;
+    void* data;
+    NAPI_OK(napi_get_typedarray_info(env, a.v[1], &t, &len, &data, nullptr, nullptr));
+    OLAP_CALL(olap_status_merge(src.data(), (int)src.size(), static_cast<uint8_t*>(data), (int64_t)len));
+    return nullptr;
+}
+
+// statusMap(stores[]) -> { keys: BigInt64Array, values: Float64Array, isInt: Uint8Array }   (getStatusMap of a computed measure)
+static napi_value StatusMap(napi_env env, napi_callback_info info) {
+    GET_ARGS();
+    auto src = store_list(env, a.v[0]);
+    int64_t count = 0;
+    OLAP_CALL(olap_status_map_export(src.data(), (int)src.size(), 0, nullptr, nullptr, nullptr, &count));
+    napi_value kbuf, vbuf, ibuf, keys, values, is_int, out;
+    void *kdata, *vdata, *idata;
+    NAPI_OK(napi_create_arraybuffer(env, (size_t)count * 8, &kdata, &kbuf));
+    NAPI_OK(napi_create_arraybuffer(env, (size_t)count * 8, &vdata, &vbuf));
+    NAPI_OK(napi_create_arraybuffer(env, (size_t)count, &idata, &ibuf));
+    OLAP_CALL(olap_status_map_export(src.data(), (int)src.size(), count, static_cast<int64_t*>(kdata), static_cast<double*>(vdata),
+                                     static_cast<uint8_t*>(idata), &count));
+    NAPI_OK(napi_create_typedarray(env, napi_bigint64_array, (size_t)count, kbuf, 0, &keys));
+    NAPI_OK(napi_create_typedarray(env, napi_float64_array, (size_t)count, vbuf, 0, &values));
+    NAPI_OK(napi_create_typedarray(env, napi_uint8_array, (size_t)count, ibuf, 0, &is_int));
+    NAPI_OK(napi_create_object(env, &out));
+    NAPI_OK(napi_set_named_property(env, out, "keys", keys));
+    NAPI_OK(napi_set_named_property(env, out, "values", values));
+    NAPI_OK(napi_set_named_property(env, out, "isInt", is_int));
+    return out;
+}
+
 static napi_value Init(napi_env env, napi_value exports) {
     const napi_property_descriptor props[] = {
         {"create", nullptr, Create, nullptr, nullptr, nullptr, napi_default, nullptr},
@@ -467,6 +545,10 @@ static napi_value Init(napi_env env, napi_value exports) {
         {"importSparse", nullptr, ImportSparse, nullptr, nullptr, nullptr, napi_default, nullptr},
         {"evaluate", nullptr, Evaluate, nullptr, nullptr, nullptr, napi_default, nullptr},
         {"evaluateToStore", nullptr, EvaluateToStore, nullptr, nullptr, nullptr, napi_default, nullptr},
+        {"regionEvalSum", nullptr, RegionEvalSum, nullptr, nullptr, nullptr, napi_default, nullptr},
+        {"regionEvalCopy", nullptr, RegionEvalCopy, nullptr, nullptr, nullptr, napi_default, nullptr},
+        {"statusMerge", nullptr, StatusMerge, nullptr, nullptr, nullptr, napi_default, nullptr},
+        {"statusMap", nullptr, StatusMap, nullptr, nullptr, nullptr, napi_default, nullptr},
     };
     napi_define_properties(env, exports, sizeof props / sizeof props[0], props);
     if (olap_init(0) != OLAP_OK) return throw_last(env);  // no CPU fallback: fail at require() time

@@ -293,6 +293,39 @@ int olap_region_copy(olap_store* dst, const olap_store* src, int ndim, const int
 int olap_eval(const char* program, olap_store* const* inputs, int n_inputs, const double* totals, int n_totals,
               double* out_host_f64, int out_type, int out_default_kind, olap_store** out_store);
 
+/* ---- computed measures over a region (Cube.getTotalForDimensionItems / getDistribution / copyMeasureData
+ * of a computed measure).  `program` is a formula as for olap_eval, without totals (t<k>); inputs[k] is the
+ * store of v<k>.  The region is that of olap_region_sum.  The formula is evaluated only at the region's cells,
+ * in double, by the same function olap_eval uses (so a cell gets the bits getData returns for it), in ONE
+ * NVRTC kernel that walks the region like region_kernel.  An empty region launches nothing. */
+/* Sum over the region's cells of the formula's value, repeats counted (region/eval-sum, one launch).
+ * NaN and +-inf propagate as in a double sum; summation order is fixed for a given region: repeated calls
+ * give the same bits. */
+int olap_region_eval_sum(const char* program, olap_store* const* inputs, int n_inputs, int ndim, const int64_t* len,
+                         const int64_t* keep_len, const int32_t* const* keep, double* out);
+/* dst.setValue(i, formula(i)) for every cell i of the region (region/eval-copy): the value rounded to
+ * Float32, canonicalised for dst's default, status byte SET / UNSET.  dst may be one of the inputs: every
+ * value is computed before its cell is written (each item list is de-duplicated first; a repeat would write
+ * the same value again).  Cells outside the region are not touched.  An int32 / uint32 target refuses the
+ * whole call, before anything is written, when a value does not survive its Float32 cell (as
+ * olap_store_set_values does), naming the first such cell in product order: a check launch, then the write. */
+int olap_region_eval_copy(olap_store* dst, const char* program, olap_store* const* inputs, int n_inputs, int ndim,
+                          const int64_t* len, const int64_t* keep_len, const int32_t* const* keep);
+
+/* ---- the status accessors of a computed measure (Cube.getStatus / getStatusMap, cube.js:368-389) ---- */
+/* getStatus: host[i] = OR over the inputs of their status byte of cell i: the plane's byte, or SET / UNSET
+ * from the values for an input without a plane (what olap_store_status reports for it).  n_cells = the
+ * stores' size.  One launch (status/merge), then the download. */
+int olap_status_merge(olap_store* const* inputs, int n, uint8_t* host, int64_t n_cells);
+/* getStatusMap: the union of the stores' set cells (by value, as olap_store_export_sparse), keys grouped by
+ * the first store in which the cell is set and ascending within a group (the insertion order of cube.js's
+ * Map).  values[j] folds the key's set values over the stores in order: the first one; then, for each later
+ * one, ToInt32(prev) | ToInt32(v) when prev is truthy (not NaN, not 0; is_int[j] = 1), else v itself
+ * (is_int[j] = 0).  Two calls, as olap_store_export_sparse: keys / values / is_int all NULL -> *count only; then
+ * all three arrays, of `capacity` >= *count entries (status/map).  A mix of NULL and non-NULL arrays is an error. */
+int olap_status_map_export(olap_store* const* stores, int n, int64_t capacity, int64_t* keys, double* values,
+                           uint8_t* is_int, int64_t* count);
+
 #ifdef __cplusplus
 }
 #endif

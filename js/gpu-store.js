@@ -163,6 +163,29 @@ class GpuStore {
     return Array.from(out);
   }
 
+  // Computed measures over a region (getTotalForDimensionItems / copyMeasureData of a computed measure): the
+  // formula is evaluated only at the region's cells, in the kernel that walks the region (no whole-cube
+  // evaluation, nothing per cell on the host).  A formula with an `x__total` variable never gets here.
+  static regionEvalSum(expression, cellNames, stores, len, keep) {
+    return native.regionEvalSum(cellProgram(expression, cellNames), stores.map((s) => s._h), len, keep);
+  }
+  static regionEvalCopy(target, expression, cellNames, stores, len, keep) {
+    native.regionEvalCopy(target._h, cellProgram(expression, cellNames), stores.map((s) => s._h), len, keep);
+  }
+
+  // getStatus / getStatusMap of a computed measure (cube.js:368-389): one kernel each.
+  static statusMerge(stores, size) {
+    const out = new Uint8Array(size);
+    native.statusMerge(stores.map((s) => s._h), out);
+    return Array.from(out);
+  }
+  static statusMap(stores) {
+    const { keys, values, isInt } = native.statusMap(stores.map((s) => s._h));
+    const out = new Map();
+    keys.forEach((k, j) => out.set(Number(k), isInt[j] ? values[j] | 0 : values[j]));
+    return out;
+  }
+
   // Batched forms used by a patched Cube to serve all measures with one launch.
   static drillUpMany(stores, oldDims, newDims, methods) {
     const maps = newDims.map((nd, i) => Int32Array.from(oldDims[i].getGroupIndexFromRootIndexMap(nd.rootAttribute)));
@@ -171,6 +194,12 @@ class GpuStore {
       .drillUp(stores.map((s) => s._h), Int32Array.from(methods, (m) => METHODS[m ?? 'sum']), lens(oldDims), lens(newDims), maps)
       .map((h, i) => stores[i]._wrap(h, size));
   }
+}
+
+function cellProgram(expression, cellNames) {
+  const slots = {};
+  cellNames.forEach((n, k) => { slots[n] = `v${k}`; });
+  return toPostfix(expression.tokens, slots);
 }
 
 module.exports = GpuStore;

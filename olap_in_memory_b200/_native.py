@@ -113,6 +113,10 @@ SIGNATURES = {
     "olap_region_sum": (C.c_int, [p_store, C.c_int, p_i64, p_i64, pp_i32, p_f64]),
     "olap_region_copy": (C.c_int, [p_store, p_store, C.c_int, p_i64, p_i64, pp_i32]),
     "olap_eval": (C.c_int, [C.c_char_p, pp_store, C.c_int, p_f64, C.c_int, C.c_void_p, C.c_int, C.c_int, pp_store]),
+    "olap_region_eval_sum": (C.c_int, [C.c_char_p, pp_store, C.c_int, C.c_int, p_i64, p_i64, pp_i32, p_f64]),
+    "olap_region_eval_copy": (C.c_int, [p_store, C.c_char_p, pp_store, C.c_int, C.c_int, p_i64, p_i64, pp_i32]),
+    "olap_status_merge": (C.c_int, [pp_store, C.c_int, C.c_void_p, C.c_int64]),
+    "olap_status_map_export": (C.c_int, [pp_store, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, p_i64]),
 }
 
 

@@ -12,6 +12,7 @@
 #include <vector>
 
 #include "../../include/olap_gpu.h"
+#include "region_walk.cuh"  // FastDiv
 
 namespace olap {
 
@@ -184,28 +185,5 @@ __device__ __forceinline__ float js_min(float a, float b) {
     if (a != a || b != b) r = canon_nan();
     return r;
 }
-
-// Division by a runtime constant without the 64-bit divide unit.
-struct FastDiv {
-    uint32_t d = 1, mul = 0, shift = 0;
-    FastDiv() {}
-    explicit FastDiv(uint32_t div) : d(div) {
-        // round-up method valid for n < 2^31
-        if (div <= 1) { mul = 0; shift = 0; return; }
-        uint32_t l = 0;
-        while ((1ull << l) < div) ++l;
-        shift = l;
-        mul = (uint32_t)(((1ull << 32) * ((1ull << l) - div)) / div + 1);
-    }
-    __host__ __device__ __forceinline__ uint32_t div(uint32_t n) const {
-        if (d == 1) return n;
-#ifdef __CUDA_ARCH__
-        uint32_t t = __umulhi(mul, n);
-#else
-        uint32_t t = (uint32_t)(((uint64_t)mul * n) >> 32);
-#endif
-        return (t + ((n - t) >> 1)) >> (shift - 1);
-    }
-};
 
 }  // namespace olap

@@ -162,8 +162,8 @@ inline bool lower_program(const char* program, Lowered& out, std::string& err) {
     return true;
 }
 
-inline std::string eval_source(const Lowered& lw, int n_inputs, int n_totals) {
-    std::ostringstream s;
+// Helpers and `olap_formula`: the same text in every kernel kind, so a cell gets the same bits in each.
+inline void formula_prelude(std::ostringstream& s, const Lowered& lw, int n_inputs, int n_totals) {
     s << "typedef long long i64;\n"
          "__device__ __forceinline__ double olap_nan() { return __longlong_as_double(0x7ff8000000000000LL); }\n"
          "__device__ __forceinline__ double olap_inf() { return __longlong_as_double(0x7ff0000000000000LL); }\n"
@@ -198,6 +198,12 @@ inline std::string eval_source(const Lowered& lw, int n_inputs, int n_totals) {
     for (int k = 0; k < n_inputs; ++k) { s << (first ? "" : ", ") << "double x" << k; first = false; }
     for (int k = 0; k < n_totals; ++k) { s << (first ? "" : ", ") << "double t" << k; first = false; }
     s << ") { return " << lw.expr << "; }\n";
+}
+
+inline std::string eval_source(const Lowered& lw, int n_inputs, int n_totals) {
+    std::ostringstream s;
+    bool first = true;
+    formula_prelude(s, lw, n_inputs, n_totals);
     s << "extern \"C\" __global__ void __launch_bounds__(256) olap_eval_kernel(";
     for (int k = 0; k < n_inputs; ++k) s << "const float* __restrict__ v" << k << ", ";
     for (int k = 0; k < n_totals; ++k) s << "double t" << k << ", ";
@@ -242,29 +248,218 @@ inline std::string eval_source(const Lowered& lw, int n_inputs, int n_totals) {
     return s.str();
 }
 
+// ---- the formula over a region (olap_region_eval_sum / olap_region_eval_copy) -------------------------
+// The region is walked by region_walk.cuh exactly as region_kernel walks it; each input is read at the same
+// offset, the formula is evaluated in double, and the value is summed (kind JIT_REGION_SUM, epilogue of
+// region_kernel's SUM) or stored into the target with setValue's element body (kind JIT_REGION_COPY).
+// A module holds each kernel for VEC 4 (128-bit accesses) and VEC 1.
+enum JitKind { JIT_EVAL = 0, JIT_REGION_SUM = 1, JIT_REGION_COPY = 2 };
+
+inline std::string region_source(const Lowered& lw, int n_inputs, int kind) {
+    std::ostringstream s;
+    s << "#include \"region_walk.cuh\"\n";
+    formula_prelude(s, lw, n_inputs, 0);
+    // vectors in flight per thread: U x n_inputs loads of VEC floats
+    const int U = n_inputs >= 4 ? 1 : (n_inputs >= 2 ? 2 : 4);
+    s << "constexpr int U = " << U << ";\n"
+         "template <int VEC, bool NC> __device__ __forceinline__ void olap_ld(const float* p, float (&x)[VEC]) {\n"
+         "  if (VEC == 4) { const float4 a = NC ? __ldcs(reinterpret_cast<const float4*>(p)) : *reinterpret_cast<const float4*>(p);\n"
+         "    x[0] = a.x; x[1 % VEC] = a.y; x[2 % VEC] = a.z; x[3 % VEC] = a.w; }\n"
+         "  else x[0] = NC ? __ldcs(p) : *p; }\n";
+    auto params = [&](std::ostringstream& o) {
+        for (int k = 0; k < n_inputs; ++k) o << ", const float* v" << k;
+    };
+    auto formula_at = [&](const char* u, const char* e) {
+        std::ostringstream o;
+        o << "olap_formula(";
+        for (int k = 0; k < n_inputs; ++k) o << (k ? ", " : "") << "(double)x" << k << "[" << u << "][" << e << "]";
+        o << ")";
+        return o.str();
+    };
+    auto loads = [&](bool nc) {
+        std::ostringstream o;
+        for (int k = 0; k < n_inputs; ++k) o << "float x" << k << "[U][VEC];\n";
+        o << "#pragma unroll\n  for (int u = 0; u < U; ++u) { if (off[u] < 0) continue;\n";
+        for (int k = 0; k < n_inputs; ++k) o << "    olap_ld<VEC, " << (nc ? "true" : "false") << ">(v" << k << " + off[u], x" << k << "[u]);\n";
+        o << "  }\n";
+        return o.str();
+    };
+    const char* walk_head =
+        "  const i64 n = w.n_vec;\n"
+        "  const i64 stride = (i64)gridDim.x * blockDim.x;\n"
+        "  for (i64 t0 = (i64)blockIdx.x * blockDim.x + threadIdx.x; t0 < n; t0 += U * stride) {\n"
+        "    i64 off[U];\n"
+        "#pragma unroll\n"
+        "    for (int u = 0; u < U; ++u) { const i64 t = t0 + u * stride; off[u] = t < n ? olap::region_offset(w, t, VEC) : -1; }\n";
+    // the last CTA of a ticketed grid: s_last in shared memory
+    const char* ticket =
+        "  __shared__ bool s_last;\n"
+        "  __threadfence();\n"
+        "  __syncthreads();\n"
+        "  if (threadIdx.x == 0) s_last = atomicAdd(ticket, 1u) == gridDim.x - 1;\n"
+        "  __syncthreads();\n";
+    if (kind == JIT_REGION_SUM) {
+        s << "__device__ __forceinline__ double olap_warp_sum(double x) {\n"
+             "#pragma unroll\n  for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);\n  return x; }\n";
+        s << "template <int VEC> __device__ __forceinline__ void region_eval_sum(const olap::RegionWalk& w";
+        params(s);
+        s << ", double* partial, unsigned* ticket, double* out) {\n"
+             "  double accs[U];\n"
+             "#pragma unroll\n  for (int u = 0; u < U; ++u) accs[u] = 0.0;\n"
+          << walk_head << loads(true)
+          << "#pragma unroll\n    for (int u = 0; u < U; ++u) { if (off[u] < 0) continue;\n"
+             "#pragma unroll\n      for (int e = 0; e < VEC; ++e) accs[u] += " << formula_at("u", "e") << "; }\n"
+             "  }\n"
+             // region_kernel's epilogue: per-CTA partials folded in a fixed order by the last CTA
+             "  __shared__ double s_sum[256 / 32];\n"
+             "  double a0 = accs[0];\n"
+             "#pragma unroll\n  for (int u = 1; u < U; ++u) a0 += accs[u];\n"
+             "  const double acc = olap_warp_sum(a0);\n"
+             "  const int wi = threadIdx.x >> 5, l = threadIdx.x & 31;\n"
+             "  if (l == 0) s_sum[wi] = acc;\n"
+             "  __shared__ bool s_last;\n"
+             "  __syncthreads();\n"
+             "  if (threadIdx.x == 0) {\n"
+             "    double a = 0.0;\n"
+             "    for (int k = 0; k < 256 / 32; ++k) a += s_sum[k];\n"
+             "    partial[blockIdx.x] = a;\n"
+             "    __threadfence();\n"
+             "    s_last = atomicAdd(ticket, 1u) == gridDim.x - 1;\n"
+             "  }\n"
+             "  __syncthreads();\n"
+             "  if (!s_last) return;\n"
+             "  double a = 0.0;\n"
+             "  for (unsigned b = threadIdx.x; b < gridDim.x; b += blockDim.x) a += ((volatile double*)partial)[b];\n"
+             "  a = olap_warp_sum(a);\n"
+             "  __syncthreads();\n"
+             "  if (l == 0) s_sum[wi] = a;\n"
+             "  __syncthreads();\n"
+             "  if (threadIdx.x == 0) {\n"
+             "    double ta = 0.0;\n"
+             "    for (int k = 0; k < 256 / 32; ++k) ta += s_sum[k];\n"
+             "    *out = ta;\n"
+             "    *ticket = 0;\n"
+             "  }\n"
+             "}\n";
+        for (int vec : {4, 1}) {
+            s << "extern \"C\" __global__ void __launch_bounds__(256, 4) olap_region_eval_sum_v" << vec
+              << "(const __grid_constant__ olap::RegionWalk w";
+            params(s);
+            s << ", double* partial, unsigned* ticket, double* out) { region_eval_sum<" << vec << ">(w";
+            for (int k = 0; k < n_inputs; ++k) s << ", v" << k;
+            s << ", partial, ticket, out); }\n";
+        }
+        return s.str();
+    }
+    // JIT_REGION_COPY.  Every cell of the (de-duplicated) region is read and written by one thread, once, so
+    // the target may be an input: the loads are plain (not .nc) and each value is computed before its cell
+    // is written.  The check kernel (integer targets) writes nothing: it finds the first cell, in product
+    // order, whose value does not survive the Float32 cell; its last CTA evaluates that cell once more and
+    // reports its offset and value.
+    s << "template <int VEC> __device__ __forceinline__ void region_eval_copy(const olap::RegionWalk& w";
+    params(s);
+    s << ", float* dst, unsigned char* st_dst, int nan_default) {\n"
+      << walk_head << loads(false)
+      << "#pragma unroll\n    for (int u = 0; u < U; ++u) { if (off[u] < 0) continue;\n"
+         "      float o[VEC]; unsigned so = 0;\n"
+         "#pragma unroll\n      for (int e = 0; e < VEC; ++e) {\n"
+         "        o[e] = olap_canon((float)" << formula_at("u", "e") << ", nan_default);\n"
+         "        so |= (unsigned)((nan_default ? o[e] == o[e] : o[e] != 0.0f) ? 2 : 1) << (8 * e); }\n"
+         "      if (VEC == 4) {\n"
+         "        *reinterpret_cast<float4*>(dst + off[u]) = make_float4(o[0], o[1 % VEC], o[2 % VEC], o[3 % VEC]);\n"
+         "        if (st_dst) *reinterpret_cast<unsigned*>(st_dst + off[u]) = so;\n"
+         "      } else {\n"
+         "        dst[off[u]] = o[0];\n"
+         "        if (st_dst) st_dst[off[u]] = (unsigned char)so;\n"
+         "      }\n"
+         "    }\n"
+         "  }\n"
+         "}\n";
+    s << "template <int VEC> __device__ __forceinline__ void region_eval_check(const olap::RegionWalk& w";
+    params(s);
+    s << ", unsigned long long* first, unsigned* ticket, i64* bad_off, double* bad_val) {\n"
+      << walk_head << loads(false)
+      << "#pragma unroll\n    for (int u = 0; u < U; ++u) { if (off[u] < 0) continue;\n"
+         "#pragma unroll\n      for (int e = 0; e < VEC; ++e) {\n"
+         "        const double r = " << formula_at("u", "e") << ";\n"
+         "        if (r == r && (double)(float)r != r) atomicMin(first, (unsigned long long)((t0 + u * stride) * VEC + e)); } }\n"
+         "  }\n"
+      << ticket
+      << "  if (!s_last || threadIdx.x != 0) return;\n"
+         "  *ticket = 0;\n"
+         "  const unsigned long long pos = atomicAdd(first, 0ull);\n"
+         "  if (pos == ~0ull) return;\n"
+         "  const i64 o = olap::region_offset(w, (i64)(pos / VEC), VEC) + (i64)(pos % VEC);\n"
+         "  *bad_off = o;\n"
+         "  *bad_val = olap_formula(";
+    for (int k = 0; k < n_inputs; ++k) s << (k ? ", " : "") << "(double)v" << k << "[o]";
+    s << ");\n}\n";
+    for (int vec : {4, 1}) {
+        s << "extern \"C\" __global__ void __launch_bounds__(256, 4) olap_region_eval_copy_v" << vec
+          << "(const __grid_constant__ olap::RegionWalk w";
+        params(s);
+        s << ", float* dst, unsigned char* st_dst, int nan_default) { region_eval_copy<" << vec << ">(w";
+        for (int k = 0; k < n_inputs; ++k) s << ", v" << k;
+        s << ", dst, st_dst, nan_default); }\n";
+        s << "extern \"C\" __global__ void __launch_bounds__(256, 4) olap_region_eval_check_v" << vec
+          << "(const __grid_constant__ olap::RegionWalk w";
+        params(s);
+        s << ", unsigned long long* first, unsigned* ticket, i64* bad_off, double* bad_val) { region_eval_check<" << vec << ">(w";
+        for (int k = 0; k < n_inputs; ++k) s << ", v" << k;
+        s << ", first, ticket, bad_off, bad_val); }\n";
+    }
+    return s.str();
+}
+
+// region_walk.cuh as text (generated by the Makefile): the in-memory header of the region kinds
+static const char kRegionWalkHeader[] =
+#include "region_walk.inc"
+    ;
+
 struct JitKernel {
     CUmodule mod = nullptr;
-    CUfunction fn = nullptr;
+    CUfunction fn = nullptr;             // JIT_EVAL: olap_eval_kernel
+    CUfunction vec4 = nullptr, vec1 = nullptr;      // region kinds: the sum or copy kernel
+    CUfunction check4 = nullptr, check1 = nullptr;  // JIT_REGION_COPY: the check pass of integer targets
 };
 
-inline int jit_get(const char* program, int n_inputs, int n_totals, JitKernel** out) {
+// CUDA source of a formula program for one kernel kind; on error `code` is set and `err` says why
+inline std::string jit_source(const char* program, int n_inputs, int n_totals, int kind, std::string& err, int* code) {
+    Lowered lw;
+    *code = OLAP_OK;
+    if (!lower_program(program, lw, err)) { *code = OLAP_E_INVALID; return ""; }
+    char buf[128];
+    if (lw.max_input >= n_inputs) {
+        snprintf(buf, sizeof buf, "formula reads input %d but only %d given", lw.max_input, n_inputs);
+        err = buf; *code = OLAP_E_INVALID; return "";
+    }
+    if (lw.max_total >= n_totals) {
+        snprintf(buf, sizeof buf, "formula reads total %d but only %d given", lw.max_total, n_totals);
+        err = buf; *code = OLAP_E_INVALID; return "";
+    }
+    return kind == JIT_EVAL ? eval_source(lw, n_inputs, n_totals) : region_source(lw, n_inputs, kind);
+}
+
+inline int jit_get(const char* program, int n_inputs, int n_totals, int kind, JitKernel** out) {
     static std::map<std::string, JitKernel> cache;
-    const std::string key = std::to_string(n_inputs) + "|" + std::to_string(n_totals) + "|" + (program ? program : "");
+    const std::string key = std::to_string(kind) + "|" + std::to_string(n_inputs) + "|" + std::to_string(n_totals) + "|" +
+                            (program ? program : "");
     auto it = cache.find(key);
     if (it != cache.end()) { *out = &it->second; return OLAP_OK; }
 
-    Lowered lw;
     std::string err;
-    if (!lower_program(program, lw, err)) return fail(OLAP_E_INVALID, "%s", err.c_str());
-    if (lw.max_input >= n_inputs) return fail(OLAP_E_INVALID, "formula reads input %d but only %d given", lw.max_input, n_inputs);
-    if (lw.max_total >= n_totals) return fail(OLAP_E_INVALID, "formula reads total %d but only %d given", lw.max_total, n_totals);
+    int code;
+    const std::string src = jit_source(program, n_inputs, n_totals, kind, err, &code);
+    if (code != OLAP_OK) return fail(code, "%s", err.c_str());
 
     JitApi& api = jit_api();
     if (!api.ok) return fail(OLAP_E_CUDA, "computed-measure JIT unavailable: %s", api.why.c_str());
 
-    const std::string src = eval_source(lw, n_inputs, n_totals);
     nvrtcProgram prog;
-    if (api.CreateProgram(&prog, src.c_str(), "olap_eval.cu", 0, nullptr, nullptr) != NVRTC_SUCCESS)
+    const char* hdr_src[] = {kRegionWalkHeader};
+    const char* hdr_name[] = {"region_walk.cuh"};
+    const int n_hdr = kind == JIT_EVAL ? 0 : 1;
+    if (api.CreateProgram(&prog, src.c_str(), "olap_eval.cu", n_hdr, n_hdr ? hdr_src : nullptr, n_hdr ? hdr_name : nullptr) != NVRTC_SUCCESS)
         return fail(OLAP_E_CUDA, "nvrtcCreateProgram failed");
     const char* opts[] = {"--gpu-architecture=sm_100a", "--std=c++17", "-lineinfo", "--fmad=false"};
     const nvrtcResult rc = api.CompileProgram(prog, 4, opts);
@@ -284,7 +479,12 @@ inline int jit_get(const char* program, int n_inputs, int n_totals, JitKernel** 
 
     JitKernel k;
     CUresult cr = api.ModuleLoadData(&k.mod, cubin.data());
-    if (cr == CUDA_SUCCESS) cr = api.ModuleGetFunction(&k.fn, k.mod, "olap_eval_kernel");
+    if (cr == CUDA_SUCCESS && kind == JIT_EVAL) cr = api.ModuleGetFunction(&k.fn, k.mod, "olap_eval_kernel");
+    const char* base = kind == JIT_REGION_SUM ? "olap_region_eval_sum_v" : "olap_region_eval_copy_v";
+    if (cr == CUDA_SUCCESS && kind != JIT_EVAL) cr = api.ModuleGetFunction(&k.vec4, k.mod, (std::string(base) + "4").c_str());
+    if (cr == CUDA_SUCCESS && kind != JIT_EVAL) cr = api.ModuleGetFunction(&k.vec1, k.mod, (std::string(base) + "1").c_str());
+    if (cr == CUDA_SUCCESS && kind == JIT_REGION_COPY) cr = api.ModuleGetFunction(&k.check4, k.mod, "olap_region_eval_check_v4");
+    if (cr == CUDA_SUCCESS && kind == JIT_REGION_COPY) cr = api.ModuleGetFunction(&k.check1, k.mod, "olap_region_eval_check_v1");
     if (cr != CUDA_SUCCESS) {
         const char* msg = "?";
         api.GetErrorString(cr, &msg);

@@ -12,8 +12,11 @@
 #include "common.cuh"
 #include "kernels_gather.cuh"
 #include "kernels_store.cuh"
+#include "region_walk.cuh"
 
 namespace olap {
+
+static_assert(kWalkMaxDims == OLAP_MAX_DIMS, "region_walk.cuh sizes its tables for OLAP_MAX_DIMS");
 
 enum RegionOp { REGION_SUM = 0, REGION_COPY = 1 };
 
@@ -29,31 +32,9 @@ struct RegionParams {
     double* out;
 };
 
-// source offset (in cells, relative to src) of work item t
-__device__ __forceinline__ int64_t region_offset(const RegionParams& p, int64_t t, int vec) {
-    const GatherParams& q = p.ix;
-    int64_t row, off;
-    if (p.big) {
-        row = t / q.IV;
-        off = (t - row * q.IV) * vec;
-        for (int d = q.nd - 1; d >= 0; --d) {
-            const int64_t r = row / q.len[d];
-            const uint32_t c = (uint32_t)(row - r * q.len[d]);
-            row = r;
-            off += q.tbl[d] ? q.tbl[d][c] : (int64_t)c * q.lin[d];
-        }
-        return off;
-    }
-    uint32_t rest = q.div_iv.div((uint32_t)t);
-    off = (int64_t)((uint32_t)t - rest * q.IV) * vec;
-    for (int d = q.nd - 1; d >= 0; --d) {
-        const uint32_t r = q.div[d].div(rest);
-        const uint32_t c = rest - r * q.len[d];
-        rest = r;
-        off += q.tbl[d] ? q.tbl[d][c] : (int64_t)c * q.lin[d];
-    }
-    return off;
-}
+// source offset (in cells, relative to src) of work item t: the walk of region_walk.cuh, which the NVRTC
+// formula region kernels (jit_eval.cuh) share
+__device__ __forceinline__ int64_t region_offset(const RegionParams& p, int64_t t, int vec) { return walk_offset(p.ix, p.big, t, vec); }
 
 // One grid-stride loop, U vectors of VEC cells in flight per thread.
 // REGION_SUM adds the raw floats in double (the status plane is never read: an unset cell holds the

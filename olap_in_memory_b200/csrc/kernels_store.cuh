@@ -292,4 +292,136 @@ __global__ void __launch_bounds__(kStoreThreads) import_sparse_kernel(float* __r
     if (st) st[k] = present_f(t, nan_default) ? OLAP_STATUS_SET : OLAP_STATUS_UNSET;
 }
 
+// ---- the status accessors of a computed measure (Cube.getStatus / getStatusMap) ---------------
+// One input store: its status plane, or (nullptr) SET / UNSET from its values.
+struct StatusIn {
+    const float* v;
+    const uint8_t* st;
+    int nan_default;
+};
+
+// getStatus: the OR over the inputs of each cell's status byte (the bytes olap_store_status reports per input)
+template <int VEC>
+__global__ void __launch_bounds__(kStoreThreads) status_merge_kernel(const StatusIn* __restrict__ in, int n,
+                                                                     uint8_t* __restrict__ out, int64_t cells) {
+    const int64_t nv = cells / VEC;
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += stride) {
+        uint32_t acc = 0;
+        for (int k = 0; k < n; ++k) {
+            const StatusIn m = in[k];
+            if (VEC == 4) {
+                if (m.st) {
+                    acc |= ld_stream_u32(m.st + i * 4);
+                } else {
+                    const float4 x = ld_stream4(m.v + i * 4);
+                    acc |= (uint32_t)(present_f(x.x, m.nan_default) ? OLAP_STATUS_SET : OLAP_STATUS_UNSET) |
+                           (uint32_t)(present_f(x.y, m.nan_default) ? OLAP_STATUS_SET : OLAP_STATUS_UNSET) << 8 |
+                           (uint32_t)(present_f(x.z, m.nan_default) ? OLAP_STATUS_SET : OLAP_STATUS_UNSET) << 16 |
+                           (uint32_t)(present_f(x.w, m.nan_default) ? OLAP_STATUS_SET : OLAP_STATUS_UNSET) << 24;
+                }
+            } else {
+                acc |= m.st ? m.st[i] : (present_f(m.v[i], m.nan_default) ? OLAP_STATUS_SET : OLAP_STATUS_UNSET);
+            }
+        }
+        if (VEC == 4) *reinterpret_cast<uint32_t*>(out + i * 4) = acc;
+        else out[i] = (uint8_t)acc;
+    }
+}
+
+// JS ToInt32 of a float32 value held in a double: NaN and +-inf give 0, then truncation and the wrap modulo 2^32.
+// A float32 of magnitude >= 2^55 is a multiple of 2^32, so ToInt32 is 0 for every one of them beyond 2^63.
+__device__ __forceinline__ int js_to_int32(double x) {
+    if (!(fabs(x) < 9223372036854775808.0)) return 0;
+    return (int)(uint32_t)(unsigned long long)(long long)x;
+}
+
+// getStatusMap of a computed measure (cube.js:374-386) for one cell: `g` = the first input in which the cell is
+// set (-1: none), `val` / `is_int` = the fold over the inputs in order: the first set value; then for each later
+// set value, ToInt32(prev) | ToInt32(v) (an int) when the previous value is truthy, else the value itself.
+__device__ __forceinline__ int status_map_cell(const StatusIn* __restrict__ in, int n, int64_t i, double& val,
+                                               uint8_t& is_int) {
+    int g = -1;
+    val = 0.0;
+    is_int = 0;
+    for (int k = 0; k < n; ++k) {
+        const float x = in[k].v[i];
+        if (!present_f(x, in[k].nan_default)) continue;
+        if (g < 0) {
+            g = k;
+            val = x;
+        } else if (val == val && val != 0.0) {
+            val = (double)(js_to_int32(val) | js_to_int32(x));
+            is_int = 1;
+        } else {
+            val = x;
+            is_int = 0;
+        }
+    }
+    return g;
+}
+
+__device__ __forceinline__ int first_set(const StatusIn* __restrict__ in, int n, int64_t i) {
+    for (int k = 0; k < n; ++k)
+        if (present_f(in[k].v[i], in[k].nan_default)) return k;
+    return -1;
+}
+
+// Ordered compaction with one bucket per input (compact_* with keys grouped by their first input): tile b's
+// count of group g goes to cnt[g * nb + b], so that one exclusive scan of cnt gives every (group, tile) its
+// first output slot.  Dynamic shared memory: n counters.
+__global__ void __launch_bounds__(256) map_count_kernel(const StatusIn* __restrict__ in, int n, int64_t cells,
+                                                        unsigned long long* __restrict__ cnt, int64_t nb) {
+    extern __shared__ unsigned int s_cnt[];
+    for (int g = threadIdx.x; g < n; g += 256) s_cnt[g] = 0;
+    __syncthreads();
+    const int64_t base = (int64_t)blockIdx.x * kCompactTile;
+    for (int k = threadIdx.x; k < kCompactTile; k += 256) {
+        const int64_t i = base + k;
+        const int g = i < cells ? first_set(in, n, i) : -1;
+        const unsigned peers = __match_any_sync(0xffffffffu, g);
+        if (g >= 0 && (threadIdx.x & 31) == __ffs(peers) - 1) atomicAdd(&s_cnt[g], (unsigned)__popc(peers));
+    }
+    __syncthreads();
+    for (int g = threadIdx.x; g < n; g += 256) cnt[(int64_t)g * nb + blockIdx.x] = s_cnt[g];
+}
+
+// Dynamic shared memory: n running counts, then 8 per-warp counts per group.
+__global__ void __launch_bounds__(256) map_write_kernel(const StatusIn* __restrict__ in, int n, int64_t cells,
+                                                        const unsigned long long* __restrict__ off, int64_t nb,
+                                                        int64_t* __restrict__ keys, double* __restrict__ vals,
+                                                        uint8_t* __restrict__ is_int) {
+    extern __shared__ unsigned int s_map[];
+    unsigned int* s_run = s_map;
+    unsigned int* s_warp = s_map + n;
+    for (int g = threadIdx.x; g < n; g += 256) s_run[g] = 0;
+    const int64_t base = (int64_t)blockIdx.x * kCompactTile;
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    for (int k0 = 0; k0 < kCompactTile; k0 += 256) {
+        for (int q = threadIdx.x; q < n * 8; q += 256) s_warp[q] = 0;
+        __syncthreads();
+        const int64_t i = base + k0 + threadIdx.x;
+        double val = 0.0;
+        uint8_t as_int = 0;
+        const int g = i < cells ? status_map_cell(in, n, i, val, as_int) : -1;
+        const unsigned peers = __match_any_sync(0xffffffffu, g);
+        if (g >= 0 && lane == __ffs(peers) - 1) s_warp[g * 8 + w] = __popc(peers);
+        __syncthreads();
+        if (g >= 0) {
+            unsigned long long pos = off[(int64_t)g * nb + blockIdx.x] + s_run[g] + __popc(peers & ((1u << lane) - 1u));
+            for (int q = 0; q < w; ++q) pos += s_warp[g * 8 + q];
+            keys[pos] = i;
+            vals[pos] = val;
+            is_int[pos] = as_int;
+        }
+        __syncthreads();
+        for (int q = threadIdx.x; q < n; q += 256) {
+            unsigned int t = 0;
+            for (int x = 0; x < 8; ++x) t += s_warp[q * 8 + x];
+            s_run[q] += t;
+        }
+        __syncthreads();
+    }
+}
+
 }  // namespace olap

@@ -9,6 +9,7 @@
 #include <array>
 #include <map>
 #include <numeric>
+#include <unordered_set>
 
 #include "common.cuh"
 #include "jit_eval.cuh"
@@ -2310,7 +2311,7 @@ int olap_eval(const char* program, olap_store* const* inputs, int n_inputs, cons
     OLAP_TRY(check_batch(inputs, n_inputs, "olap_eval", &size));
     OLAP_TRY(ensure_ctx());
     JitKernel* k = nullptr;
-    OLAP_TRY(jit_get(program, n_inputs, n_totals, &k));
+    OLAP_TRY(jit_get(program, n_inputs, n_totals, JIT_EVAL, &k));
 
     float* out32 = nullptr;
     uint8_t* st_out = nullptr;
@@ -2363,6 +2364,285 @@ int olap_eval(const char* program, olap_store* const* inputs, int n_inputs, cons
         OLAP_CUDA(cudaStreamSynchronize(g.stream));
     }
     return OLAP_OK;
+}
+
+// ---- computed measures over a region: getTotalForDimensionItems / copyMeasureData ------------------
+namespace {
+
+static int formula_inputs(const char* what, const char* program, olap_store* const* inputs, int n, int64_t* size) {
+    if (!program) return fail(OLAP_E_INVALID, "%s: null program", what);
+    return check_batch(inputs, n, what, size);
+}
+
+// VEC 4 when the plan and the planes of every input (and of the target) allow it
+static int region_vec_all(const RegionPlan& plan, olap_store* const* in, int n, const olap_store* dst) {
+    int vec = 4;
+    const int64_t c = plan.const_off;
+    for (int k = 0; k < n; ++k) vec = std::min(vec, region_vec(plan, in[k]->values + c, in[k]->values + c, nullptr));
+    if (dst) vec = std::min(vec, region_vec(plan, dst->values + c, dst->values + c, dst->status ? dst->status + c : nullptr));
+    return vec;
+}
+
+// the index fields of region_params as the RegionWalk the NVRTC kernels take
+static int region_walk_of(const RegionPlan& plan, int VEC, TablePack& t, RegionWalk& w) {
+    RegionParams p{};
+    OLAP_TRY(region_params(plan, VEC, t, p));
+    w = RegionWalk{};
+    w.nd = p.ix.nd;
+    for (int d = 0; d < p.ix.nd; ++d) {
+        w.len[d] = p.ix.len[d];
+        w.div[d] = p.ix.div[d];
+        w.tbl[d] = p.ix.tbl[d];
+        w.lin[d] = p.ix.lin[d];
+    }
+    w.IV = p.ix.IV;
+    w.div_iv = p.ix.div_iv;
+    w.n_vec = p.ix.n_vec;
+    w.big = p.big;
+    return OLAP_OK;
+}
+
+static int jit_launch(CUfunction fn, int blocks, std::vector<void*>& args) {
+    const CUresult cr = jit_api().LaunchKernel(fn, blocks, 1, 1, 256, 1, 1, 0, (CUstream)g.stream, args.data(), nullptr);
+    if (cr != CUDA_SUCCESS) {
+        const char* msg = "?";
+        jit_api().GetErrorString(cr, &msg);
+        return fail(OLAP_E_CUDA, "launching the formula region kernel failed: %s", msg);
+    }
+    LAUNCHED();
+    return OLAP_OK;
+}
+
+}  // namespace
+
+int olap_region_eval_sum(const char* program, olap_store* const* inputs, int n_inputs, int ndim, const int64_t* len,
+                         const int64_t* keep_len, const int32_t* const* keep, double* out) {
+    if (!out) return fail(OLAP_E_INVALID, "olap_region_eval_sum: null argument");
+    int64_t size = 0;
+    OLAP_TRY(formula_inputs("olap_region_eval_sum", program, inputs, n_inputs, &size));
+    RegionPlan plan;
+    OLAP_TRY(plan_region("olap_region_eval_sum", size, ndim, len, keep_len, keep, &plan));
+    OLAP_TRY(ensure_ctx());
+    *out = 0.0;
+    if (plan.cells == 0) {
+        begin_op();
+        end_op("region/eval-sum");
+        return finish_op();
+    }
+    JitKernel* k = nullptr;
+    OLAP_TRY(jit_get(program, n_inputs, 0, JIT_REGION_SUM, &k));
+    begin_op();
+    const int VEC = region_vec_all(plan, inputs, n_inputs, nullptr);
+    RegionWalk w;
+    TablePack t;
+    OLAP_TRY(region_walk_of(plan, VEC, t, w));
+    const int blocks = grid_for(w.n_vec, 256);
+    void* scratch;
+    OLAP_TRY(dev_alloc(&scratch, (size_t)blocks * 8 + 16));
+    double* partial = static_cast<double*>(scratch);
+    double* dout = partial + blocks;
+    unsigned int* ticket = reinterpret_cast<unsigned int*>(dout + 1);
+    OLAP_CUDA(cudaMemsetAsync(ticket, 0, 4, g.stream));
+    std::vector<const float*> ptrs(n_inputs);
+    std::vector<void*> args{&w};
+    for (int q = 0; q < n_inputs; ++q) { ptrs[q] = inputs[q]->values + plan.const_off; args.push_back(&ptrs[q]); }
+    args.push_back(&partial); args.push_back(&ticket); args.push_back(&dout);
+    KERNELS_BEGIN();
+    OLAP_TRY(jit_launch(VEC == 4 ? k->vec4 : k->vec1, blocks, args));
+    end_op("region/eval-sum");
+    double host = 0.0;
+    OLAP_CUDA(cudaMemcpyAsync(&host, dout, 8, cudaMemcpyDeviceToHost, g.stream));
+    OLAP_TRY(t.release());
+    OLAP_TRY(dev_free(scratch));
+    OLAP_CUDA(cudaStreamSynchronize(g.stream));
+    *out = host;
+    return finish_op();
+}
+
+int olap_region_eval_copy(olap_store* dst, const char* program, olap_store* const* inputs, int n_inputs, int ndim,
+                          const int64_t* len, const int64_t* keep_len, const int32_t* const* keep) {
+    if (!dst) return fail(OLAP_E_INVALID, "olap_region_eval_copy: null store");
+    int64_t size = 0;
+    OLAP_TRY(formula_inputs("olap_region_eval_copy", program, inputs, n_inputs, &size));
+    if (dst->size != size) return fail(OLAP_E_INVALID, "olap_region_eval_copy: stores of %lld and %lld cells", (long long)dst->size, (long long)size);
+    if (ndim < 0 || ndim > OLAP_MAX_DIMS) return fail(OLAP_E_INVALID, "olap_region_eval_copy: at most %d dimensions", OLAP_MAX_DIMS);
+    // Each list de-duplicated, first occurrences in order (the multiplicity axis becomes one item): every cell is
+    // then read and written by one thread, once, so the target may be an input.  A repeat writes the value it
+    // wrote before, so the planes end as those of the setValue per combination.
+    std::vector<std::vector<int32_t>> uniq(ndim);
+    std::vector<const int32_t*> kp(ndim, nullptr);
+    std::vector<int64_t> kl(ndim, 0);
+    for (int d = 0; d < ndim; ++d) {
+        if (!keep || !keep[d]) continue;
+        if (!keep_len || keep_len[d] < 0) return fail(OLAP_E_INVALID, "olap_region_eval_copy: dimension %d has no list length", d);
+        std::unordered_set<int32_t> seen;
+        for (int64_t j = 0; j < keep_len[d]; ++j)
+            if (seen.insert(keep[d][j]).second) uniq[d].push_back(keep[d][j]);
+        // an empty list stays a list (of no items): data() of an empty vector may be NULL, which means "whole axis"
+        static const int32_t no_items = 0;
+        kp[d] = uniq[d].empty() ? &no_items : uniq[d].data();
+        kl[d] = (int64_t)uniq[d].size();
+    }
+    RegionPlan plan;
+    OLAP_TRY(plan_region("olap_region_eval_copy", size, ndim, len, kl.data(), kp.data(), &plan));
+    OLAP_TRY(ensure_ctx());
+    // the derived flag stays as it is, as for olap_region_copy: every byte written is  set ? SET : UNSET
+    if (plan.cells == 0) {
+        begin_op();
+        end_op("region/eval-copy");
+        return finish_op();
+    }
+    JitKernel* k = nullptr;
+    OLAP_TRY(jit_get(program, n_inputs, 0, JIT_REGION_COPY, &k));
+    begin_op();
+    const int VEC = region_vec_all(plan, inputs, n_inputs, dst);
+    RegionWalk w;
+    TablePack t;
+    OLAP_TRY(region_walk_of(plan, VEC, t, w));
+    const int blocks = grid_for(w.n_vec, 256);
+    std::vector<const float*> ptrs(n_inputs);
+    std::vector<void*> args{&w};
+    for (int q = 0; q < n_inputs; ++q) { ptrs[q] = inputs[q]->values + plan.const_off; args.push_back(&ptrs[q]); }
+    KERNELS_BEGIN();
+    if (strict_ints(dst)) {
+        // olap_store_set_values refuses the whole call when a value would not survive its Float32 cell: a check
+        // pass finds the first such cell in product order (and its value) before anything is written
+        struct { unsigned long long first; int64_t off; double val; unsigned int ticket; } host;
+        void* scratch;
+        OLAP_TRY(dev_alloc(&scratch, sizeof host));
+        char* b = static_cast<char*>(scratch);
+        unsigned long long* first = reinterpret_cast<unsigned long long*>(b);
+        int64_t* bad_off = reinterpret_cast<int64_t*>(b + 8);
+        double* bad_val = reinterpret_cast<double*>(b + 16);
+        unsigned int* ticket = reinterpret_cast<unsigned int*>(b + 24);
+        OLAP_CUDA(cudaMemsetAsync(first, 0xff, 8, g.stream));
+        OLAP_CUDA(cudaMemsetAsync(ticket, 0, 4, g.stream));
+        std::vector<void*> cargs = args;
+        cargs.push_back(&first); cargs.push_back(&ticket); cargs.push_back(&bad_off); cargs.push_back(&bad_val);
+        OLAP_TRY(jit_launch(VEC == 4 ? k->check4 : k->check1, blocks, cargs));
+        OLAP_CUDA(cudaMemcpyAsync(&host, scratch, sizeof host, cudaMemcpyDeviceToHost, g.stream));
+        OLAP_TRY(dev_free(scratch));
+        OLAP_CUDA(cudaStreamSynchronize(g.stream));
+        if (host.first != ~0ull) {
+            end_op("region/eval-copy");
+            OLAP_TRY(t.release());
+            return lossy_error(dst, plan.const_off + host.off, host.val);
+        }
+    }
+    float* dv = dst->values + plan.const_off;
+    uint8_t* ds = dst->status ? dst->status + plan.const_off : nullptr;
+    int nan_default = dst->default_kind;
+    args.push_back(&dv); args.push_back(&ds); args.push_back(&nan_default);
+    OLAP_TRY(jit_launch(VEC == 4 ? k->vec4 : k->vec1, blocks, args));
+    end_op("region/eval-copy");
+    OLAP_TRY(t.release());
+    return finish_op();
+}
+
+// ---- the status accessors of a computed measure: Cube.getStatus / getStatusMap --------------------
+namespace {
+static int status_inputs(const char* what, olap_store* const* s, int n, int64_t* size, TablePack& t, size_t* o_in) {
+    if (!s || n < 1) return fail(OLAP_E_INVALID, "%s: at least one store expected", what);
+    std::vector<StatusIn> in(n);
+    for (int k = 0; k < n; ++k) {
+        if (!s[k]) return fail(OLAP_E_INVALID, "%s: null store", what);
+        if (s[k]->size != s[0]->size) return fail(OLAP_E_INVALID, "%s: stores of one call must have the same size", what);
+        in[k] = StatusIn{s[k]->values, s[k]->status, s[k]->default_kind};
+    }
+    *size = s[0]->size;
+    *o_in = t.add(in.data(), sizeof(StatusIn) * n);
+    return OLAP_OK;
+}
+}  // namespace
+
+int olap_status_merge(olap_store* const* inputs, int n, uint8_t* host, int64_t n_cells) {
+    TablePack t;
+    size_t o_in = 0;
+    int64_t size = 0;
+    OLAP_TRY(status_inputs("olap_status_merge", inputs, n, &size, t, &o_in));
+    if (size != n_cells) return fail(OLAP_E_INVALID, "value length is invalid: %lld !== %lld", (long long)size, (long long)n_cells);
+    if (n_cells && !host) return fail(OLAP_E_INVALID, "olap_status_merge: null argument");
+    OLAP_TRY(ensure_ctx());
+    begin_op();
+    if (n_cells == 0) {
+        end_op("status/merge");
+        return finish_op();
+    }
+    bool vec4 = n_cells % 4 == 0;
+    for (int k = 0; k < n; ++k)
+        vec4 &= ((reinterpret_cast<uintptr_t>(inputs[k]->values) & 15) | (reinterpret_cast<uintptr_t>(inputs[k]->status) & 3)) == 0;
+    OLAP_TRY(t.upload());
+    void* tmp;
+    OLAP_TRY(dev_alloc(&tmp, (size_t)n_cells));
+    KERNELS_BEGIN();
+    if (vec4) status_merge_kernel<4><<<grid_for(n_cells / 4, kStoreThreads), kStoreThreads, 0, g.stream>>>(t.ptr<StatusIn>(o_in), n, (uint8_t*)tmp, n_cells);
+    else status_merge_kernel<1><<<grid_for(n_cells, kStoreThreads), kStoreThreads, 0, g.stream>>>(t.ptr<StatusIn>(o_in), n, (uint8_t*)tmp, n_cells);
+    LAUNCHED();
+    end_op("status/merge");
+    OLAP_TRY(copy_d2h(host, tmp, (size_t)n_cells));
+    OLAP_TRY(t.release());
+    OLAP_TRY(dev_free(tmp));
+    return finish_op();
+}
+
+int olap_status_map_export(olap_store* const* stores, int n, int64_t capacity, int64_t* keys, double* values,
+                           uint8_t* is_int, int64_t* count) {
+    if (!count) return fail(OLAP_E_INVALID, "olap_status_map_export: null argument");
+    const bool fill = keys != nullptr;
+    if ((values != nullptr) != fill || (is_int != nullptr) != fill)
+        return fail(OLAP_E_INVALID, "olap_status_map_export: keys, values and is_int must be all NULL (count) or all given (fill)");
+    *count = 0;
+    TablePack t;
+    size_t o_in = 0;
+    int64_t size = 0;
+    OLAP_TRY(status_inputs("olap_status_map_export", stores, n, &size, t, &o_in));
+    OLAP_TRY(ensure_ctx());
+    if (size == 0) {
+        begin_op();
+        end_op("status/map");
+        return finish_op();
+    }
+    OLAP_TRY(t.upload());
+    const int64_t nb = ceil_div(size, kCompactTile);
+    const int64_t nc = (int64_t)n * nb;
+    void* cnt;
+    OLAP_TRY(dev_alloc(&cnt, (size_t)(nc + 1) * 8));
+    unsigned long long* d_cnt = (unsigned long long*)cnt;
+    const StatusIn* in = t.ptr<StatusIn>(o_in);
+    begin_op();
+    KERNELS_BEGIN();
+    map_count_kernel<<<(unsigned)nb, 256, (size_t)n * 4, g.stream>>>(in, n, size, d_cnt, nb);
+    LAUNCHED();
+    compact_scan_kernel<<<1, 1024, 0, g.stream>>>(d_cnt, nc, d_cnt + nc);
+    LAUNCHED();
+    unsigned long long total = 0;
+    OLAP_CUDA(cudaMemcpyAsync(&total, d_cnt + nc, 8, cudaMemcpyDeviceToHost, g.stream));
+    OLAP_CUDA(cudaStreamSynchronize(g.stream));
+    *count = (int64_t)total;
+    const bool write = fill && total && (int64_t)total <= capacity;
+    void *dk = nullptr, *dv = nullptr, *di = nullptr;
+    if (write) {
+        OLAP_TRY(dev_alloc(&dk, (size_t)total * 8));
+        OLAP_TRY(dev_alloc(&dv, (size_t)total * 8));
+        OLAP_TRY(dev_alloc(&di, (size_t)total));
+        map_write_kernel<<<(unsigned)nb, 256, (size_t)n * 9 * 4, g.stream>>>(in, n, size, d_cnt, nb, (int64_t*)dk, (double*)dv, (uint8_t*)di);
+        LAUNCHED();
+    }
+    end_op("status/map");  // every path that launched closes the op here
+    int rc = OLAP_OK;
+    if (fill && (int64_t)total > capacity)
+        rc = fail(OLAP_E_INVALID, "olap_status_map_export: capacity %lld < %llu keys", (long long)capacity, total);
+    if (write) {
+        OLAP_TRY(copy_d2h(keys, dk, (size_t)total * 8));
+        OLAP_TRY(copy_d2h(values, dv, (size_t)total * 8));
+        OLAP_TRY(copy_d2h(is_int, di, (size_t)total));
+        OLAP_TRY(dev_free(dk));
+        OLAP_TRY(dev_free(dv));
+        OLAP_TRY(dev_free(di));
+    }
+    OLAP_TRY(t.release());
+    OLAP_TRY(dev_free(cnt));
+    return rc == OLAP_OK ? finish_op() : rc;
 }
 
 }  // extern "C"

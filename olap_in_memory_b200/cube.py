@@ -130,6 +130,19 @@ def _region(dimensions, dimensionsFilter, check_measures):
     return lens, keep
 
 
+def _formula_inputs(store_cls, member, computedMeasures, storedMeasures, measureId):
+    """(expression, cell names, their stores) of a computed measure when the store class has `member` (the device
+    forms of the region queries and status accessors) and the formula reads at least one cell; else None, and the
+    caller keeps its host code.  Formulas with an `x__total` variable were rejected by _check_readable before."""
+    if getattr(store_cls, member, None) is None:
+        return None
+    expression = computedMeasures[measureId]
+    cell_names = [n for n in expression.variables() if "__total" not in n]
+    if not cell_names:
+        return None
+    return expression, cell_names, [storedMeasures[n] for n in cell_names]
+
+
 def _region_lists(lens, keep):
     return [np.arange(n) if k is None else np.asarray(k, dtype=np.int64) for n, k in zip(lens, keep)]
 
@@ -338,6 +351,9 @@ class Cube:
         if measureId in self.storedMeasures:
             return self.storedMeasures[measureId]._dataMap
         if measureId in self.computedMeasures:
+            status_map = getattr(self._store_cls, "statusMap", None)
+            if status_map is not None:
+                return status_map(list(self.storedMeasures.values())) if self.storedMeasures else {}
             # cube.js:374-386: union of the stored measures' keys in first-seen order; a key seen before
             # with a truthy value gets  previous | value  (JS ToInt32 bitwise OR), else the value itself
             result = {}
@@ -357,6 +373,9 @@ class Cube:
         if measureId in self.storedMeasures:
             return self.storedMeasures[measureId].status
         if measureId in self.computedMeasures:
+            fused = _formula_inputs(self._store_cls, "statusMerge", self.computedMeasures, self.storedMeasures, measureId)
+            if fused is not None:
+                return self._store_cls.statusMerge(fused[2], self.storeSize)
             merged = None
             for name in self.computedMeasures[measureId].variables():
                 if "__total" in name:
@@ -482,6 +501,9 @@ class Cube:
         lens, keep = region
         if measureId in self.storedMeasures:
             return self.storedMeasures[measureId].regionSum(lens, keep)
+        fused = _formula_inputs(self._store_cls, "regionEvalSum", self.computedMeasures, self.storedMeasures, measureId)
+        if fused is not None:
+            return self._store_cls.regionEvalSum(*fused, lens, keep)
         return _region_sum_f64(np.asarray(self.getData(measureId), dtype=np.float64), lens, keep)
 
     def getDistribution(self, measureId, dimensionsFilter=None):
@@ -502,6 +524,10 @@ class Cube:
         target = self.storedMeasures[targetMeasureId]
         if sourceMeasureId in self.storedMeasures:
             target.regionCopy(self.storedMeasures[sourceMeasureId], lens, keep)
+            return
+        fused = _formula_inputs(self._store_cls, "regionEvalCopy", self.computedMeasures, self.storedMeasures, sourceMeasureId)
+        if fused is not None:
+            self._store_cls.regionEvalCopy(target, *fused, lens, keep)
         else:
             _region_set_f64(target, np.asarray(self.getData(sourceMeasureId), dtype=np.float64), lens, keep)
 

@@ -444,6 +444,9 @@ class ShardedCube:
         lens, keep = region
         if measureId in self.storedMeasures:
             local = self.storedMeasures[measureId].regionSum(lens, keep)
+        elif (fused := _cube._formula_inputs(self._store_cls, "regionEvalSum", self.computedMeasures, self.storedMeasures,
+                                             measureId)) is not None:
+            local = self._store_cls.regionEvalSum(*fused, lens, keep)
         else:
             local = _cube._region_sum_f64(np.asarray(self.getLocalData(measureId), dtype=np.float64), lens, keep)
         device = self._store_cls.DEVICE if self.world > 1 else None
@@ -468,6 +471,9 @@ class ShardedCube:
         target = self.storedMeasures[targetMeasureId]
         if sourceMeasureId in self.storedMeasures:
             target.regionCopy(self.storedMeasures[sourceMeasureId], lens, keep)
+        elif (fused := _cube._formula_inputs(self._store_cls, "regionEvalCopy", self.computedMeasures, self.storedMeasures,
+                                             sourceMeasureId)) is not None:
+            self._store_cls.regionEvalCopy(target, *fused, lens, keep)
         else:
             _cube._region_set_f64(target, np.asarray(self.getLocalData(sourceMeasureId), dtype=np.float64), lens, keep)
 

@@ -256,6 +256,60 @@ class GpuStore:
         N.check(N.lib().olap_region_copy(self._h, src._h, nd, len_arr, keep_len, ptrs))
         del alive
 
+    # ---- computed measures over a region, status of a computed measure (Cube) -----------
+    @staticmethod
+    def regionEvalSum(expression, cell_names, stores, lens, keep):
+        """Sum of a formula of cell variables over keep[0] x ... x keep[-1] (repeats counted): ONE kernel that
+        evaluates it only at the region's cells (include/olap_gpu.h, olap_region_eval_sum)."""
+        program = GpuStore._program(expression, cell_names, [])
+        alive, nd, len_arr, keep_len, ptrs = GpuStore._region_args(lens, keep)
+        out = C.c_double()
+        N.check(N.lib().olap_region_eval_sum(program.encode(), N.store_array([s._h for s in stores]), len(stores), nd,
+                                             len_arr, keep_len, ptrs, C.byref(out)))
+        del alive
+        return out.value
+
+    @staticmethod
+    def regionEvalCopy(target, expression, cell_names, stores, lens, keep):
+        """target.setValue(i, formula(i)) for every cell i of the region, in place (olap_region_eval_copy); the
+        target may be one of the formula's inputs."""
+        program = GpuStore._program(expression, cell_names, [])
+        alive, nd, len_arr, keep_len, ptrs = GpuStore._region_args(lens, keep)
+        N.check(N.lib().olap_region_eval_copy(target._h, program.encode(), N.store_array([s._h for s in stores]),
+                                              len(stores), nd, len_arr, keep_len, ptrs))
+        del alive
+
+    @staticmethod
+    def statusMerge(stores, size):
+        """Status bytes of a computed measure: the OR of its inputs' bytes, one kernel (olap_status_merge)."""
+        out = np.empty(size, dtype=np.uint8)
+        N.check(N.lib().olap_status_merge(N.store_array([s._h for s in stores]), len(stores), out.ctypes.data, size))
+        return out.tolist()
+
+    @staticmethod
+    def statusMap_arrays(stores):
+        """(keys int64, values float64, is_int uint8) of the status map of a computed measure over `stores`, in
+        the order of the dict (olap_status_map_export)."""
+        handles = N.store_array([s._h for s in stores])
+        count = C.c_int64()
+        N.check(N.lib().olap_status_map_export(handles, len(stores), 0, None, None, None, C.byref(count)))
+        keys = np.empty(count.value, dtype=np.int64)
+        values = np.empty(count.value, dtype=np.float64)
+        is_int = np.empty(count.value, dtype=np.uint8)
+        if count.value:
+            N.check(N.lib().olap_status_map_export(handles, len(stores), count.value, keys.ctypes.data, values.ctypes.data,
+                                                   is_int.ctypes.data, C.byref(count)))
+        return keys, values, is_int
+
+    @staticmethod
+    def statusMap(stores):
+        """Cube.getStatusMap of a computed measure: {cell: value} with ints where the fold ORed values."""
+        keys, values, is_int = GpuStore.statusMap_arrays(stores)
+        vals = values.tolist()
+        for j in np.flatnonzero(is_int).tolist():
+            vals[j] = int(vals[j])
+        return dict(zip(keys.tolist(), vals))
+
     # ---- single-store forms of the transforms ------------------------------------
     def reorder(self, oldDimensions, newDimensions):
         return GpuStore.reorder_many([self], oldDimensions, newDimensions)[0]
